@@ -6,7 +6,7 @@ GPU, obstacle set ISRR_2H: one step = uniform-grid build + r-ball neighbour tabl
 point validity (K6) + validity of every stored edge (K7: column classify + per-edge kernel).  metric = collision-checked edges/s
 (the NN-queries/s figure of the same step is reported beside it).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 N > 1: launched by torch.distributed.run, one rank per GPU.  The headline line is WEAK scaling -- the
 sample set grows to N x 1M (replicated on every GPU, stripe order), rank g owns the query columns
@@ -402,6 +402,32 @@ def parity_check(job, rank, world, windows=4, width=256):
     return checked
 
 
+def dump_outputs(job, out_dir, sample_cols=32768):
+    """What the last timed step left for its caller, as DIR/<name>.npy (float64; float32 for bits): this rank's
+    colptr and point validity in full, and rowval / nzval / edge validity of the entries of a fixed, seeded sample
+    of columns (the full table is ~28M entries per 1M columns).  Integers are exact in float64."""
+    import torch
+    from mpb200 import sharding
+    os.makedirs(out_dir, exist_ok=True)
+    colptr, rowval, nzval, words = sharding.table_device_tensors(job.NN.table)
+    cp = colptr.cpu().numpy()
+    ncols = len(cp) - 1
+    cols = np.sort(np.random.Generator(np.random.PCG64(SEED)).choice(ncols, min(sample_cols, ncols), replace=False))
+    # 0-based positions of every entry of the sampled columns
+    idx = np.concatenate([np.arange(cp[j] - 1, cp[j + 1] - 1) for j in cols])
+    ti = torch.from_numpy(idx).to(colptr.device)
+    e_bits = (words[ti >> 6] >> (ti & 63)) & 1
+    # the step enqueues K6 with its bits left on the device; fetching them re-runs the same pure per-sample test
+    p_bits = np.unpackbits(job.NN.points_free(job.CC, job.SS).view(np.uint8), bitorder="little")[:ncols]
+    arrays = {"colptr": cp.astype(np.float64), "point_free": p_bits.astype(np.float32),
+              "sample_columns": cols.astype(np.float64),
+              "sample_rowval": rowval[ti].cpu().numpy().astype(np.float64),
+              "sample_nzval": nzval[ti].cpu().numpy(),
+              "sample_edge_free": e_bits.cpu().numpy().astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def allreduce_max_sum(vals_max, vals_sum, world):
     import torch
     import torch.distributed as dist
@@ -459,7 +485,13 @@ def main():
     ap.add_argument("--no-secondary", action="store_true", help="skip the C3/C4/C5 secondary block (N = 1) and the MC leg")
     ap.add_argument("--scaling", default="weak", choices=["weak", "strong"],
                     help="headline line: weak (N x 1M samples) or strong (1M samples in total); the other one is still reported as a sub-object")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (rank 0's columns) to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the b200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -501,6 +533,8 @@ def main():
     sampler = ClockSampler(local)
     total_ms, launches, t_wall = timed_steps(job, lib, stream, flush, args.steps, args.warmup, world, sampler, phases)
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(job, args.dump_outputs)
     nnz = job.nnz
     (total_ms_max,), (edges_all,) = allreduce_max_sum([total_ms], [float(nnz)], world)
     per_rank = None
