@@ -24,6 +24,11 @@ NN = mpb200.MetricNN(V); NN.set_query_range(2000, 5000); NN.precompute(0.03); NN
 # d >= 4: tensor-core prefilter + CUDA-core fallback dimension
 for d in (6, 16):
     V = rng.random((1500, d)); NN = mpb200.MetricNN(V); NN.precompute(0.9 if d == 6 else 1.4); NN.close()
+# d >= 4 shard with unaligned ends (one-sided tensor-core sweep, estimated cap), and 500 samples pairwise farther
+# apart than r (empty probe: cap = 0, the count-only sweep decides colptr)
+V = rng.random((3000, 6)); NN = mpb200.MetricNN(V); NN.set_query_range(37, 2461); NN.precompute(0.6); NN.close()
+idx = rng.choice(3 ** 6, size=500, replace=False)
+V = ((idx[:, None] // 3 ** np.arange(6)) % 3) * 0.5; NN = mpb200.MetricNN(V); NN.precompute(0.45); NN.close()
 # boxes
 B = mpb200.PointRobotNDBoxes([mpb200.BoxBounds(np.array([[0.2, 0.4], [0.2, 0.4], [0.0, 1.0]]))])
 V = rng.random((3000, 3)); NN = mpb200.MetricNN(V); NN.precompute(0.1)

@@ -58,6 +58,12 @@ def uniform_samples(N, d, seed):
     return np.random.Generator(np.random.PCG64(seed)).random((N, d))
 
 
+def lattice_cloud(rng, n, d, step, lo, hi):
+    """points on the lattice step * Z^d inside [lo, hi]^d (exactly representable: differences and squares are exact)"""
+    k0, k1 = int(np.ceil(lo / step)), int(np.floor(hi / step))
+    return rng.integers(k0, k1 + 1, size=(n, d)).astype(np.float64) * step
+
+
 def random_hyperboxes(M, d, seed, init=0.1, goal=0.9):
     """SURVEY 8(d) C3: centre U[0,1)^d, half-widths U[0.05,0.25), clipped to the cube; boxes
     containing init*1 or goal*1 are resampled."""

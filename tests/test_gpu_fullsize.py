@@ -91,12 +91,6 @@ def test_full_size_c4_lq_tables_and_edges(gpu, orc):
     NN.close()
 
 
-def _lattice_cloud(rng, n, d, step, lo, hi):
-    """points on the lattice step * Z^d inside [lo, hi]^d (exactly representable: differences and squares are exact)"""
-    k0, k1 = int(np.ceil(lo / step)), int(np.floor(hi / step))
-    return rng.integers(k0, k1 + 1, size=(n, d)).astype(np.float64) * step
-
-
 @pytest.mark.parametrize("offset", [0.0, 1000.0, -3.0e4])
 def test_k3_tensor_core_band_adversarial_10d(gpu, orc, offset):
     """d = 10, compact cloud (the tensor-core prefilter is in use): partners planted EXACTLY at the radius along
@@ -105,7 +99,7 @@ def test_k3_tensor_core_band_adversarial_10d(gpu, orc, offset):
     mp = gpu
     rng = np.random.Generator(np.random.PCG64(2718))
     d, step = 10, 1.0 / 32
-    base = _lattice_cloud(rng, 700, d, step, 0.0, 0.65)
+    base = fx.lattice_cloud(rng, 700, d, step, 0.0, 0.65)
     r = 10.0 / 32                                          # |(6,8,0..)|/32 = |(5,5,5,5,0..)|/32 = |(4,4,4,4,4,4,2,0..)|/32
     dirs = np.zeros((3, d))
     dirs[0, :2] = (6, 8)

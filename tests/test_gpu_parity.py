@@ -149,8 +149,10 @@ def test_k3_k4_high_dim_rball_matches_oracle(gpu, orc, d, N):
 
 
 def test_k3_prefilter_band_has_no_false_negatives(gpu, orc):
-    """adversarial for the FP32 prefilter: pairs EXACTLY at the radius, large coordinate offsets
-    (FP32 conversion error >> the gap to the radius), shard ranges"""
+    """adversarial for the FP32 CUDA-core prefilter: pairs EXACTLY at the radius, large coordinate offsets
+    (FP32 conversion error >> the gap to the radius), shard ranges.  The cloud is wide against r (2 delta / r^2
+    ~ 0.8 - 1), so the build takes the CUDA-core sweep, not the tensor cores; the tensor-core form of this test is
+    the c-band cases of test_gpu_k3_paths.py."""
     mp = gpu
     rng = np.random.Generator(np.random.PCG64(17))
     d = 5
@@ -312,7 +314,9 @@ def test_fused_build_checked_equals_separate_calls(gpu, orc, checker):
 
 def test_k3_single_sweep_slab_overflow_falls_back(gpu, orc):
     """the slab capacity is sized from a probe of the first 2048 columns; a dense cluster among
-    later indices overflows it and the build must fall back to the two-sweep fill"""
+    later indices overflows it and the build must fall back to the two-sweep fill.  The cluster far away makes
+    the cloud wide against r (2 delta / r^2 ~ 2.3), so this exercises the FP32 CUDA-core sweep; overflow after a
+    tensor-core sweep is the d-overflow cases of test_gpu_k3_paths.py."""
     mp = gpu
     rng = np.random.Generator(np.random.PCG64(5))
     d = 5
