@@ -75,6 +75,7 @@ int64_t mpb200_launch_count(void);
 #define MPB200_OP_POINTS 1 /* mpb200_points_free */
 #define MPB200_OP_EDGES 2  /* mpb200_edges_free / mpb200_lq_edges_free */
 #define MPB200_OP_OTHER 3  /* mpb200_mc_collision_probability */
+#define MPB200_OP_PLAN 4   /* mpb200_gmt_plan: phase 1 = the planning kernel */
 double mpb200_last_ms(int phase);
 double mpb200_last_ms_of(int op, int phase);
 
@@ -360,6 +361,53 @@ int mpb200_pipe_peak(int kind, double *ops_per_s);
  * fill kernel visits them, constant data.  This is what the reference's CSC output format costs on the device before
  * any neighbour work: the floor the fill kernel's time is compared with, next to the plain-copy HBM peak. */
 int mpb200_table_write_floor(const mpb200_table *t, double *ms);
+
+/* ---- planning on the device: group-marching FMT* (GMT*; Ichter, Schmerling & Pavone 2017) -------------------
+ * Plans over tables and validity bits that are already on the device, so nothing N-sized crosses PCIe on the way in.
+ * Inputs: samples 1..N of s; fwd (DF: column z holds the x with an edge z -> x); bwd (DB: column x holds the y with
+ * an edge y -> x and its cost) with its edge bits (the last mpb200_edges_free / _lq_ / _car_ result on bwd); the
+ * point bits of s (the last mpb200_points_free) when checkpts != 0, else every sample counts as free; a goal mask;
+ * a width w = lambda * r.
+ * State: C (cost), A (parent, 0 = none), status W (unvisited) / H (open) / closed.  Initially only init is in H, C = 0.
+ * Each iteration:
+ *   1. H empty: failed.  Else thr = min_{y in H} C[y] + w (one FP64 add), group G = { y in H : C[y] <= thr }.
+ *   2. G holds a goal vertex: solved; the result is the goal vertex of G with the smallest (C, index).
+ *   3. candidates X = { x in column g of DF for some g in G : x in W, free(x) }.
+ *   4. every x in X, against the state at the start of the iteration: among the entries e of column x of DB whose
+ *      row y is in H (G included), none -> skip x; else e* = the first in storage order minimising C[y] + nzval[e]
+ *      (one FP64 add); count one check (and one in checks_in_bounds when V[y] lies in the space bounds); if the
+ *      edge bit of e* is set: A[x] = y, C[x] = that cost, x joins H_new.
+ *   5. G becomes closed, H_new joins H.
+ * At w = 0 with no two open vertices of equal cost, G is the vertex FMT*'s heap would dequeue: tree, cost, path and
+ * check count equal fmtstar's.  Every output is a function of sets: identical for every run and launch geometry.
+ * One cooperative kernel runs the whole loop (no host round trip per iteration); MPB200_GMT_GRID=<blocks> forces its
+ * grid size (clamped to the co-resident maximum).
+ * Rejected with MPB200_EARG: tables built from another sample set or over a query range other than [0, N), missing
+ * or stale edge bits on bwd, checkpts without full-range point bits of s. */
+typedef struct {
+    const mpb200_table *fwd;        /* DF */
+    const mpb200_table *bwd;        /* DB, with current edge bits */
+    const uint64_t *goal_bits;      /* host BitVector chunks, ceil(N/64) words: goal mask */
+    int64_t init;                   /* 1-based */
+    double width;                   /* w = lambda * r, >= 0 */
+    int32_t checkpts;               /* 0: every sample counts as free */
+    const mpb200_space_desc *space; /* optional (NULL: checks_in_bounds = 0): bounds for checks_in_bounds */
+} mpb200_gmt_desc;
+typedef struct {
+    int32_t solved;
+    int32_t grid_blocks;        /* blocks of the cooperative launch */
+    int64_t goal;               /* 1-based goal vertex reached, 0 when failed */
+    double cost;                /* C[goal], +inf when failed */
+    int64_t iterations;         /* groups expanded */
+    int64_t expansions;         /* sum of |G| over them */
+    int64_t checks;             /* edge-bit lookups (step 4) */
+    int64_t checks_in_bounds;   /* of those, with V[y] inside the space bounds */
+    int64_t path_len;           /* vertices init .. goal, 0 when failed */
+} mpb200_gmt_result;
+/* path: path_len 1-based vertices init .. goal, written only when path_len <= path_cap (path may be NULL when
+ * path_cap == 0); tree (N int64, parents, 1-based, 0 = none) and costs (N f64) may be NULL.  Waits for the result. */
+int mpb200_gmt_plan(const mpb200_samples *s, const mpb200_gmt_desc *desc, mpb200_gmt_result *res, int64_t *path,
+                    int64_t path_cap, int64_t *tree, double *costs);
 
 #ifdef __cplusplus
 }

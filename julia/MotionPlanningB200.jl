@@ -350,4 +350,43 @@ function table_union_transpose(a::Ptr{Void}, b::Ptr{Void})
     out[], nnz[]
 end
 
+# ---- GMT* on the device: mpb200_gmt_plan over tables and bits that never leave HBM ----------------------------
+# C layouts of mpb200_gmt_desc / mpb200_gmt_result (include/mpb200.h).
+immutable GmtDescC
+    fwd::Ptr{Void}
+    bwd::Ptr{Void}
+    goal_bits::Ptr{UInt64}
+    init::Int64
+    width::Float64
+    checkpts::Int32
+    space::Ptr{SpaceDescC}
+end
+immutable GmtResultC
+    solved::Int32
+    grid_blocks::Int32
+    goal::Int64
+    cost::Float64
+    iterations::Int64
+    expansions::Int64
+    checks::Int64
+    checks_in_bounds::Int64
+    path_len::Int64
+end
+"""gmtstar over device tables: s the sample set, tF / tB the forward / backward table handles (tB with its edge bits,
+the same handle twice for a symmetric metric), goal a BitVector over the samples, w = lambda * r.  Points bits must have
+been computed on s (mpb200_points_free) unless checkpts = false.  Returns (result, path, tree, costs)."""
+function gmtstar_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::BitVector, w::Float64, sd::SpaceDesc;
+                      checkpts = true)
+    N = length(goal)
+    path = Vector{Int64}(N); tree = Vector{Int64}(N); costs = Vector{Float64}(N)
+    res = Ref{GmtResultC}()
+    desc = Ref(GmtDescC(tF, tB, pointer(goal.chunks), 1, w, Int32(checkpts),
+                        Base.unsafe_convert(Ptr{SpaceDescC}, sd.c)))        # goal and sd stay rooted by the arguments
+    check(ccall((:mpb200_gmt_plan, LIB), Cint,
+                (Ptr{Void}, Ref{GmtDescC}, Ref{GmtResultC}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}),
+                s.h, desc, res, path, N, tree, costs))
+    r = res[]
+    r, path[1:r.path_len], tree, costs
+end
+
 end # module

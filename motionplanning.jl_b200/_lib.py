@@ -47,8 +47,18 @@ class McResult(ctypes.Structure):
     _fields_ = [("s1", c_dbl), ("s2", c_dbl), ("s0", c_dbl), ("n", c_i64), ("hits", c_i64)]
 
 
+class GmtDesc(ctypes.Structure):
+    _fields_ = [("fwd", c_vp), ("bwd", c_vp), ("goal_bits", c_vp), ("init", c_i64), ("width", c_dbl),
+                ("checkpts", c_i32), ("space", P(SpaceDesc))]
+
+
+class GmtResult(ctypes.Structure):
+    _fields_ = [("solved", c_i32), ("grid_blocks", c_i32), ("goal", c_i64), ("cost", c_dbl), ("iterations", c_i64),
+                ("expansions", c_i64), ("checks", c_i64), ("checks_in_bounds", c_i64), ("path_len", c_i64)]
+
+
 # every symbol include/mpb200.h declares: name -> (restype, argtypes)
-OP_TABLE, OP_POINTS, OP_EDGES, OP_OTHER = 0, 1, 2, 3  # mpb200_last_ms_of operation kinds
+OP_TABLE, OP_POINTS, OP_EDGES, OP_OTHER, OP_PLAN = 0, 1, 2, 3, 4  # mpb200_last_ms_of operation kinds
 
 SIGNATURES = {
     "mpb200_init": (ctypes.c_int, [ctypes.c_int]),
@@ -106,6 +116,7 @@ SIGNATURES = {
     "mpb200_car_edges_free": (ctypes.c_int, [c_vp, c_vp, ctypes.c_int32, c_dbl, c_dbl, c_vp, P(SpaceDesc), c_vp, P(c_i64)]),
     "mpb200_car_motions_free": (ctypes.c_int, [ctypes.c_int32, c_dbl, c_dbl, c_vp, c_vp, c_i64, c_vp, P(SpaceDesc), c_vp, P(c_i64)]),
     "mpb200_lq_motions_free": (ctypes.c_int, [c_vp, c_dbl, c_vp, c_vp, c_i64, c_vp, P(SpaceDesc), c_vp, P(c_i64)]),
+    "mpb200_gmt_plan": (ctypes.c_int, [c_vp, P(GmtDesc), P(GmtResult), c_vp, c_i64, c_vp, c_vp]),
 }
 
 _lib = None

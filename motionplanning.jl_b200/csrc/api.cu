@@ -65,6 +65,11 @@ void *cache_take(size_t bytes, size_t *cap) {
 
 size_t cache_parked_bytes() { return g_cached_bytes; }
 
+uint64_t next_serial() {
+    static uint64_t n = 0;
+    return ++n;
+}
+
 void cache_release_all() {
     for (const Block &b : g_blocks) cudaFree(b.p);
     g_blocks.clear();
@@ -448,6 +453,7 @@ int mpb200_inball_build(mpb200_samples *s, double r, mpb200_table **table, int64
     t->edge_bits_valid = false;  // bits of an earlier build do not describe the new table
     t->src_N = s->N;
     t->src_d = s->d;
+    t->src_serial = s->serial;
     int rc;
     if (s->N == 0) {
         rc = t->colptr.reserve(sizeof(int64_t));
@@ -800,6 +806,7 @@ int mpb200_points_free(const mpb200_samples *s_, const mpb200_obstacles *o, cons
     cudaStream_t st = ctx().stream;
     const int64_t n = s->q1 - s->q0;  // this process's shard of the samples (all of them by default)
     const size_t words = (size_t)ceil_div(n, 64);
+    s->point_bits_valid = false;
     if (int rc = s->point_bits.reserve(sizeof(uint64_t) * (words + 1))) return rc;
     phase_bank(MPB200_OP_POINTS);
     phase_mark(0);
@@ -808,6 +815,7 @@ int mpb200_points_free(const mpb200_samples *s_, const mpb200_obstacles *o, cons
     if (int rc = points_free_device(s->V.as<double>() + s->q0 * s->d, n, s->d, o, ss, s->point_bits.as<uint32_t>(), nullptr,
                                     s->pt_order_valid ? s->pt_order.as<int>() : nullptr))
         return rc;
+    s->point_bits_valid = s->q0 == 0 && s->q1 == s->N;
     phase_mark(1);
     phases_collect(1);
     if (bitchunks) {  // NULL: asynchronous, the bits stay on the device (stream-ordered with later calls)
@@ -952,6 +960,7 @@ int mpb200_lq_inball_build(mpb200_samples *s, const mpb200_lq *lq, double r, mpb
     tF->edge_bits_valid = tB->edge_bits_valid = false;
     tF->src_N = tB->src_N = s->N;
     tF->src_d = tB->src_d = s->d;
+    tF->src_serial = tB->src_serial = s->serial;
     int rc = lq->general ? lqg_inball_build(s, lq, r, tF, tB) : lq_inball_build(s, lq, r, tF, tB);
     if (rc) {
         if (freshF) mpb200_table_destroy(tF);

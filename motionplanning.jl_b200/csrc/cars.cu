@@ -735,7 +735,7 @@ static int finish_table(mpb200_table *out, const mpb200_table *cand, const mpb20
         MPB_LAUNCHED();
     }
     out->nnz = nnz; out->ncols = nc; out->col0 = cand->col0; out->r = r; out->euclid = false;
-    out->src_N = s->N; out->src_d = s->d; out->edge_bits_valid = false; out->has_order = false;
+    out->src_N = s->N; out->src_d = s->d; out->src_serial = s->serial; out->edge_bits_valid = false; out->has_order = false;
     return 0;
 }
 

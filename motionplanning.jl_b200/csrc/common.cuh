@@ -13,7 +13,7 @@ namespace mpb {
 
 constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 constexpr int kMaxPhases = 8;
-constexpr int kBanks = 4;  // separate phase-event banks: MPB200_OP_TABLE / _POINTS / _EDGES / _OTHER
+constexpr int kBanks = 5;  // separate phase-event banks: MPB200_OP_TABLE / _POINTS / _EDGES / _OTHER / _PLAN
 
 struct Context {
     bool ready = false;
@@ -75,6 +75,7 @@ struct DevBuf {
 };
 
 size_t cache_parked_bytes();  // device bytes parked in the block cache (free for the next reserve)
+uint64_t next_serial();       // process-unique id of a new sample set
 
 // timing phases: phase_begin(0) ... phase_end(0) record events on the launching stream
 void phase_bank(int op);               // select the event bank of the operation that starts now
@@ -116,9 +117,11 @@ struct mpb200_table {
     int64_t edge_bits_nnz = 0;
     int64_t src_N = -1;            // the sample set the table was built from (rowval addresses its samples)
     int src_d = 0;
+    uint64_t src_serial = 0;       // ... and its serial
 };
 
 struct mpb200_samples {
+    uint64_t serial = mpb::next_serial();  // tells tables built from this set from those built from another of equal size
     int64_t N = 0;
     int d = 0;
     int64_t q0 = 0, q1 = 0;
@@ -137,6 +140,7 @@ struct mpb200_samples {
     mpb::DevBuf scan_tmp;    // scan block sums
     mpb::DevBuf q_order;     // int32: cell-order positions owned by this shard (+ scratch)
     mpb::DevBuf point_bits;  // uint64 ceil(N/64): last mpb200_points_free result
+    bool point_bits_valid = false;  // point_bits hold the validity of all N samples (the last call covered [0, N))
     mpb::DevBuf aux;         // small per-build constants (e.g. the centring vector of the tensor-core path)
     // CUDA graph of the launch-bound front half of a grid build (K1 + count + scans), replayed
     // while the launch parameters (sizes, radius, buffer addresses) stay the same

@@ -192,7 +192,7 @@ __global__ void max_len_kernel(const int64_t *__restrict__ p1, const int64_t *__
 
 static int copy_meta(const mpb200_table *src, mpb200_table *dst) {
     dst->ncols = src->ncols; dst->col0 = src->col0; dst->r = src->r; dst->euclid = src->euclid;
-    dst->src_N = src->src_N; dst->src_d = src->src_d; dst->edge_bits_valid = false; dst->has_order = false;
+    dst->src_N = src->src_N; dst->src_d = src->src_d; dst->src_serial = src->src_serial; dst->edge_bits_valid = false; dst->has_order = false;
     if (src->has_order && src->ncols > 0) {  // same columns: the cell-order visiting list stays valid
         if (int rc = dst->col_order.reserve(sizeof(int) * (size_t)(src->ncols + 1))) return rc;
         MPB_CUDA(cudaMemcpyAsync(dst->col_order.p, src->col_order.p, sizeof(int) * (size_t)src->ncols, cudaMemcpyDeviceToDevice, ctx().stream));

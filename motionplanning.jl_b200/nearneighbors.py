@@ -342,6 +342,14 @@ class MetricNN(SampleSet):
         least k entries, keeps the k nearest of each (mpb200_table_knn) and forms the mutual neighbourhoods
         (mpb200_table_union_transpose).  Afterwards knn / knnF / knnB / mutualknn* are column views.
         Returns (knn cache, mutual cache); self.r is the radius of the last build (every stored neighbour is within it)."""
+        r = self.build_knn(k, r0, grow, max_rounds)
+        self.cache_knn = ImmutableNNC(self.fetch_table(self.table_knn, "knn"), float(r))
+        self.cache_mknn = ImmutableNNC(self.fetch_table(self.table_mknn, "mknn"), float(r))
+        return self.cache_knn, self.cache_mknn
+
+    def build_knn(self, k, r0=None, grow=1.3, max_rounds=40):
+        """Device-only part of precompute_knn: the k-nearest table `table_knn` and the mutual table `table_mknn` stay in
+        HBM.  Returns the radius of the last r-ball build."""
         N = len(self)
         k = min(int(k), N - 1)
         if k < 1:
@@ -363,9 +371,7 @@ class MetricNN(SampleSet):
         _table_knn(self.table, k, self.table_knn)
         _table_union_transpose(self.table_knn, self.table_knn, self.table_mknn)
         self.k = k
-        self.cache_knn = ImmutableNNC(self.fetch_table(self.table_knn, "knn"), float(r))
-        self.cache_mknn = ImmutableNNC(self.fetch_table(self.table_mknn, "mknn"), float(r))
-        return self.cache_knn, self.cache_mknn
+        return r
 
     def car_edges_free(self, CC, SS, fetch=True, table=None):
         return _car_edges_free(self, table if table is not None else self.table, CC, SS, fetch)
@@ -426,6 +432,15 @@ class QuasiMetricNN(SampleSet):
         """k-nearest connections under the steering cost: forward / backward cost-ball tables with a growing cost
         radius (from r0) until every column holds k entries, then the k cheapest of each and the mutual forward
         neighbourhoods  knnF(v) U { w : v in knnB(w) }.  Returns (knnF, knnB, mutualF) caches."""
+        r = self.build_knn(k, r0, grow, max_rounds)
+        self.cache_knnF = ImmutableNNC(self.fetch_table(self.table_knnF, "knnF"), float(r))
+        self.cache_knnB = ImmutableNNC(self.fetch_table(self.table_knnB, "knnB"), float(r))
+        self.cache_mknnF = ImmutableNNC(self.fetch_table(self.table_mknnF, "mknnF"), float(r))
+        return self.cache_knnF, self.cache_knnB, self.cache_mknnF
+
+    def build_knn(self, k, r0, grow=1.3, max_rounds=30):
+        """Device-only part of precompute_knn: `table_knnF`, `table_knnB` and `table_mknnF` stay in HBM.  Returns the
+        cost radius of the last build."""
         N = len(self)
         k = min(int(k), N - 1)
         r = float(r0)
@@ -444,10 +459,7 @@ class QuasiMetricNN(SampleSet):
         _table_knn(self.tableB, k, self.table_knnB)
         _table_union_transpose(self.table_knnF, self.table_knnB, self.table_mknnF)
         self.k = k
-        self.cache_knnF = ImmutableNNC(self.fetch_table(self.table_knnF, "knnF"), float(r))
-        self.cache_knnB = ImmutableNNC(self.fetch_table(self.table_knnB, "knnB"), float(r))
-        self.cache_mknnF = ImmutableNNC(self.fetch_table(self.table_mknnF, "mknnF"), float(r))
-        return self.cache_knnF, self.cache_knnB, self.cache_mknnF
+        return r
 
     def car_edges_free(self, CC, SS, fetch=True, table=None):
         return _car_edges_free(self, table if table is not None else self.tableB, CC, SS, fetch)

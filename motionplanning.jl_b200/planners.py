@@ -274,3 +274,111 @@ def fmtstar(P, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, init_id
     }
     P.solution = MPSolution(P.status, float(C[z - 1]), time.perf_counter() - t_start, meta)
     return P.status, P.solution.cost, P.solution.elapsed
+
+
+def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1, init_idx=1, checkpts=True, seed=0,
+            k=None):
+    """Group-marching FMT* (GMT*; Ichter, Schmerling & Pavone 2017) planned on the device -> (status, cost, elapsed)
+
+    Sets the problem up exactly as fmtstar does (radius, steering, sample_free, goal mask), builds the tables and
+    validity bits with the device-only calls and plans over them in one cooperative kernel (mpb200_gmt_plan): each
+    iteration expands, all at once, every open vertex whose cost is within lam * r of the cheapest one.  No table
+    crosses PCIe; the path, tree and costs come back.  At lam = 0 (and no two open vertices of equal cost) the tree,
+    path, cost and "collision_checks" equal fmtstar's.  Specification: include/mpb200.h, DESIGN.md section 10b."""
+    from . import _lib
+    import ctypes
+
+    t_start = time.perf_counter()
+    N = len(P.V) if N is None else N
+    P.CC.count = 0
+    if connections not in ("R", "K"):
+        raise ValueError("Connection type must be radial (:R) or k-nearest (:K)")
+    if not lam >= 0:
+        raise ValueError("lam must be a non-negative number")
+    knn_mode = connections == "K"
+    SS, CC = P.SS, P.CC
+    if r > 0:
+        setup_steering(SS, r)
+    if not states_free(P.init, CC, SS)[0]:
+        P.status = "failed"
+        P.solution = MPSolution(P.status, math.inf, time.perf_counter() - t_start, {})
+        return math.inf
+    free_volume_ub = sample_free(P, N - len(P.V), ensure_goal_ct=ensure_goal_ct, seed=seed) if N > len(P.V) else volume(SS)
+    NN = P.V
+    V = NN.V
+    if r == 0:
+        r = fmt_radius(N, SS.dim, rm, free_volume_ub)
+        setup_steering(SS, r)
+    if k is None:
+        k = min(int(math.ceil((2 * rm) ** SS.dim * (math.e / SS.dim) * math.log(N))), N - 1)
+    if not np.all(V[init_idx - 1] == P.init):
+        raise RuntimeError("P.V[init_idx] must be the init state (fmt.jl:48-66)")
+
+    # ---- the same tables and bits as fmtstar(edge_checks="table"), left on the device -------------------
+    lq = isinstance(SS.dist, LinearQuadratic)
+    car = is_car_metric(SS.dist)
+    if knn_mode and (lq or (car and not SS.dist.symmetric)):
+        r = NN.build_knn(k, r)
+        setup_steering(SS, r)
+        NN.r = r
+        DF, DB = NN.table_mknnF, NN.table_knnB
+        (NN.car_edges_free if car else NN.lq_edges_free)(CC, SS, fetch=False, table=DB)
+    elif knn_mode and car:
+        r = NN.build_knn(k, r)
+        setup_steering(SS, r)
+        NN.r = r
+        DF, DB = NN.table_mknn, NN.table_knn
+        NN.car_edges_free(CC, SS, fetch=False, table=DB)
+    elif knn_mode:
+        NN.build_knn(k)
+        DF, DB = NN.table_mknn, NN.table_knn
+        NN.edges_free(DB, CC, SS, fetch=False)
+    elif car and SS.dist.symmetric:
+        NN.build_table(r)
+        DF = DB = NN.table
+        NN.car_edges_free(CC, SS, fetch=False)
+    elif car or lq:
+        NN.build_tables(r)
+        DF, DB = NN.tableF, NN.tableB
+        (NN.car_edges_free if car else NN.lq_edges_free)(CC, SS, fetch=False)
+    else:
+        NN.build_table_checked(r, CC, SS)
+        DF = DB = NN.table
+    lookups_before = CC.count
+    CC.count = 0
+    if checkpts:
+        NN.points_free(CC, SS, fetch=False)
+    goal_chunks = np.zeros((N + 63) // 64 * 8, dtype=np.uint8)
+    packed = np.packbits(goal_mask(V, P.goal, SS), bitorder="little")
+    goal_chunks[:len(packed)] = packed
+    goal_chunks = goal_chunks.view(np.uint64)
+
+    space = SS.desc()
+    desc = _lib.GmtDesc(DF.h, DB.h, _lib.ptr(goal_chunks), init_idx, float(lam) * float(r), int(bool(checkpts)),
+                        ctypes.pointer(space))
+    res = _lib.GmtResult()
+    tree = np.empty(N, dtype=np.int64)
+    C = np.empty(N, dtype=np.float64)
+    path = np.empty(N, dtype=np.int64)
+    lib = _lib.lib()
+    _lib.check(lib.mpb200_gmt_plan(NN.handle(), ctypes.byref(desc), ctypes.byref(res), _lib.ptr(path), N,
+                                   _lib.ptr(tree), _lib.ptr(C)))
+    device_ms = lib.mpb200_last_ms_of(_lib.OP_PLAN, 0)
+    solved = bool(res.solved)
+    sol = [int(v) for v in path[:res.path_len]]
+    # fmtstar counts a Euclidean check only when y lies in the state bounds (the lazy checker's segment count)
+    checks = int(res.checks) if (lq or car) else int(res.checks_in_bounds)
+    P.status = "solved" if solved else "failed"
+    CC.count = checks
+    cost = float(res.cost)
+    meta = {
+        "radius_multiplier": rm, "collision_checks": checks, "num_samples": N, "cost": cost,
+        "cumcost": [float(C[v - 1]) for v in sol], "planner": "GMTstar", "solved": solved, "tree": tree, "path": sol,
+        "r": r, "precomputed_edge_checks": int(lookups_before), "edge_checks": "table",
+        "connections": connections, "k": (k if knn_mode else None), "device_edge_batches": 0,
+        "lambda": lam, "iterations": int(res.iterations), "expansions": int(res.expansions), "device_ms": device_ms,
+        "costs": C, "checks": int(res.checks), "checks_in_bounds": int(res.checks_in_bounds),
+        "grid_blocks": int(res.grid_blocks),
+    }
+    P.solution = MPSolution(P.status, cost, time.perf_counter() - t_start, meta)
+    return P.status, P.solution.cost, P.solution.elapsed
