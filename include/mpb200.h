@@ -409,6 +409,35 @@ typedef struct {
 int mpb200_gmt_plan(const mpb200_samples *s, const mpb200_gmt_desc *desc, mpb200_gmt_result *res, int64_t *path,
                     int64_t path_cap, int64_t *tree, double *costs);
 
+/* Lazy GMT*: the same plan without edge bits.  Step 4 reads
+ *      if is_free_motion(V[y], V[x], CC, SS): A[x] = y, C[x] = that cost, x joins H_new
+ * with the motion check evaluated inside the planning kernel, on e* only; everything else (the decision point, the
+ * argmin, the counters) is as above, so for the same tables the result equals mpb200_gmt_plan's over bits computed for
+ * the same obstacles, byte for byte.  The motion check is the one the matching edge pass runs: a straight segment
+ * (as mpb200_edges_free), the optimal LQ trajectory (as mpb200_lq_edges_free, steering horizon r) or the car path
+ * (as mpb200_car_edges_free).  *segment_checks (may be NULL) = segment tests those checks ran, each preceded by the
+ * bounds test of its first waypoint and stopping at the first failure, the last waypoint never bounds-checked: the
+ * increment of the reference's CC.count.  For straight segments it equals checks_in_bounds.
+ * desc->space is required (the space of the motion check and of checks_in_bounds).  The edge bits of bwd are never
+ * read, required or changed.  Rejected with MPB200_EARG: everything mpb200_gmt_plan rejects but the edge-bit check;
+ * NULL edges or obstacles, an unknown kind; no space; a car kind with d != 3, an unknown car kind, turning radius or
+ * speed not positive and finite; an LQ kind without a system, with a d that does not match it, or r not positive and
+ * finite; an obstacle / workspace combination the matching *_edges_free rejects.  One launch per plan. */
+#define MPB200_GMT_EDGES_STRAIGHT 0   /* as mpb200_edges_free     */
+#define MPB200_GMT_EDGES_LQ       1   /* as mpb200_lq_edges_free  */
+#define MPB200_GMT_EDGES_CAR      2   /* as mpb200_car_edges_free */
+typedef struct {
+    int32_t kind;                       /* MPB200_GMT_EDGES_* */
+    const mpb200_obstacles *obstacles;
+    const mpb200_lq *lq;                /* kind LQ */
+    double r;                           /* kind LQ: steering horizon, the r mpb200_lq_edges_free takes */
+    int32_t car_kind;                   /* kind CAR: MPB200_CAR_REEDS_SHEPP / MPB200_CAR_DUBINS */
+    double turning_radius, speed;       /* kind CAR */
+} mpb200_gmt_edges;
+int mpb200_gmt_plan_lazy(const mpb200_samples *s, const mpb200_gmt_desc *desc, const mpb200_gmt_edges *edges,
+                         mpb200_gmt_result *res, int64_t *segment_checks, int64_t *path, int64_t path_cap,
+                         int64_t *tree, double *costs);
+
 #ifdef __cplusplus
 }
 #endif

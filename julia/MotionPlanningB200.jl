@@ -389,4 +389,37 @@ function gmtstar_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::BitVec
     r, path[1:r.path_len], tree, costs
 end
 
+# C layout of mpb200_gmt_edges (include/mpb200.h): the motion check lazy GMT* runs on the one entry each candidate uses
+const GMT_EDGES_STRAIGHT = Int32(0)
+const GMT_EDGES_LQ = Int32(1)
+const GMT_EDGES_CAR = Int32(2)
+immutable GmtEdgesC
+    kind::Int32
+    obstacles::Ptr{Void}
+    lq::Ptr{Void}
+    r::Float64
+    car_kind::Int32
+    turning_radius::Float64
+    speed::Float64
+end
+"""gmtstar_b200 without edge bits (mpb200_gmt_plan_lazy): the planning kernel runs is_free_motion(V[y], V[x]) itself on
+the entry it would have looked up.  edges = GmtEdgesC(GMT_EDGES_STRAIGHT, obstacles, C_NULL, 0.0, 0, 0.0, 0.0), or
+GMT_EDGES_LQ with the LQ handle and the steering horizon r, or GMT_EDGES_CAR with the car kind, turning radius and
+speed.  tB needs no edge bits, and a new obstacle set replans over the same tables.  Returns (result, path, tree, costs,
+segment tests run)."""
+function gmtstar_lazy_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::BitVector, w::Float64, sd::SpaceDesc,
+                           edges::GmtEdgesC; checkpts = true)
+    N = length(goal)
+    path = Vector{Int64}(N); tree = Vector{Int64}(N); costs = Vector{Float64}(N)
+    res = Ref{GmtResultC}(); segs = Ref{Int64}(0)
+    desc = Ref(GmtDescC(tF, tB, pointer(goal.chunks), 1, w, Int32(checkpts),
+                        Base.unsafe_convert(Ptr{SpaceDescC}, sd.c)))
+    check(ccall((:mpb200_gmt_plan_lazy, LIB), Cint,
+                (Ptr{Void}, Ref{GmtDescC}, Ref{GmtEdgesC}, Ref{GmtResultC}, Ref{Int64}, Ptr{Int64}, Int64, Ptr{Int64},
+                 Ptr{Float64}),
+                s.h, desc, Ref(edges), res, segs, path, N, tree, costs))
+    r = res[]
+    r, path[1:r.path_len], tree, costs, segs[]
+end
+
 end # module

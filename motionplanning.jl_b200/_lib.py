@@ -57,6 +57,14 @@ class GmtResult(ctypes.Structure):
                 ("expansions", c_i64), ("checks", c_i64), ("checks_in_bounds", c_i64), ("path_len", c_i64)]
 
 
+class GmtEdges(ctypes.Structure):
+    _fields_ = [("kind", c_i32), ("obstacles", c_vp), ("lq", c_vp), ("r", c_dbl), ("car_kind", c_i32),
+                ("turning_radius", c_dbl), ("speed", c_dbl)]
+
+
+GMT_EDGES_STRAIGHT, GMT_EDGES_LQ, GMT_EDGES_CAR = 0, 1, 2  # mpb200_gmt_edges.kind
+
+
 # every symbol include/mpb200.h declares: name -> (restype, argtypes)
 OP_TABLE, OP_POINTS, OP_EDGES, OP_OTHER, OP_PLAN = 0, 1, 2, 3, 4  # mpb200_last_ms_of operation kinds
 
@@ -117,6 +125,8 @@ SIGNATURES = {
     "mpb200_car_motions_free": (ctypes.c_int, [ctypes.c_int32, c_dbl, c_dbl, c_vp, c_vp, c_i64, c_vp, P(SpaceDesc), c_vp, P(c_i64)]),
     "mpb200_lq_motions_free": (ctypes.c_int, [c_vp, c_dbl, c_vp, c_vp, c_i64, c_vp, P(SpaceDesc), c_vp, P(c_i64)]),
     "mpb200_gmt_plan": (ctypes.c_int, [c_vp, P(GmtDesc), P(GmtResult), c_vp, c_i64, c_vp, c_vp]),
+    "mpb200_gmt_plan_lazy": (ctypes.c_int, [c_vp, P(GmtDesc), P(GmtEdges), P(GmtResult), P(c_i64), c_vp, c_i64, c_vp,
+                                            c_vp]),
 }
 
 _lib = None

@@ -197,6 +197,7 @@ int lq_motions_free_device(const mpb200_lq *lq, double r, const double *dA, cons
                            const mpb200_obstacles *o, const mpb200_space_desc *ss, uint8_t *d_out,
                            unsigned long long *d_checks);
 
+int car_args(int32_t kind, double rturn, double speed);
 int car_extract_xy_device(const double *dV3, int64_t N, double *dV2);
 int car_inball_device(const mpb200_samples *s, const mpb200_table *cand, int kind, double rturn, double r, double chopval,
                       mpb200_table *tF, mpb200_table *tB, DevBuf &work, DevBuf &scan_tmp);
@@ -1097,12 +1098,6 @@ int mpb200_close_points(const mpb200_obstacles *o, const double *p_aos, const do
 }
 
 // ---- chopped-metric car spaces --------------------------------------------------------------------------------
-static int car_args(int32_t kind, double rturn, double speed) {
-    MPB_CHECK_ARG(kind == MPB200_CAR_REEDS_SHEPP || kind == MPB200_CAR_DUBINS, "kind must be MPB200_CAR_REEDS_SHEPP or MPB200_CAR_DUBINS");
-    MPB_CHECK_ARG(rturn > 0 && rturn < std::numeric_limits<double>::infinity(), "turning radius must be positive");
-    MPB_CHECK_ARG(speed > 0 && speed < std::numeric_limits<double>::infinity(), "speed must be positive");
-    return MPB200_OK;
-}
 int mpb200_car_inball_build(mpb200_samples *s, int32_t kind, double turning_radius, double r, double chopval,
                             mpb200_table **tableF, mpb200_table **tableB, int64_t *nnzF, int64_t *nnzB) {
     MPB_REQUIRE_INIT();

@@ -16,7 +16,9 @@
 #include "common.cuh"
 #include "predicates.cuh"
 #include "scan.cuh"
+#include "gmt.cuh"
 #include <algorithm>
+#include <limits>
 
 namespace mpb {
 
@@ -708,6 +710,13 @@ car_steer_kernel(const double *__restrict__ A, const double *__restrict__ Bv, in
 // ---- host side -------------------------------------------------------------------------------------------------
 int make_space(const mpb200_space_desc *ss, int d_state, SpaceDev *out, int *dw);
 
+int car_args(int32_t kind, double rturn, double speed) {
+    MPB_CHECK_ARG(kind == MPB200_CAR_REEDS_SHEPP || kind == MPB200_CAR_DUBINS, "kind must be MPB200_CAR_REEDS_SHEPP or MPB200_CAR_DUBINS");
+    MPB_CHECK_ARG(rturn > 0 && rturn < std::numeric_limits<double>::infinity(), "turning radius must be positive");
+    MPB_CHECK_ARG(speed > 0 && speed < std::numeric_limits<double>::infinity(), "speed must be positive");
+    return MPB200_OK;
+}
+
 int car_extract_xy_device(const double *dV3, int64_t N, double *dV2) {
     if (N == 0) return 0;
     const unsigned g = (unsigned)std::min<int64_t>(ceil_div(N, 256), (int64_t)ctx().sm_count * 8);
@@ -839,6 +848,33 @@ int car_steer_device(int kind, double rturn, double speed, const double *dA, con
     car_steer_kernel<<<grid, 128, 0, ctx().stream>>>(dA, dB, n, kind, rturn, speed, d_cost, d_nseg, d_segs);
     MPB_LAUNCHED();
     return 0;
+}
+
+// lazy GMT*: step 4 runs the car motion check of car_edges_free_kernel on the winning entry, on one lane
+template <int KIND>
+struct GmtCarEdge {
+    static constexpr bool kLazy = true;
+    int kind;
+    double rturn, speed;
+    SpaceDev S;
+    const double *T;
+    int M;
+    __device__ bool operator()(const GmtArgs &a, long long, int y, int x, GmtCtl *ctl) const {
+        double v[3], w[3];
+        gmt_endpoints<3>(a, y, x, v, w);
+        int nchk = 0;
+        const bool ok = car::motion_free<KIND>(kind, rturn, speed, S, T, M, v, w, &nchk);
+        gmt_count_segments(ctl, nchk);
+        return ok;
+    }
+};
+
+int gmt_lazy_car(const GmtArgs &a, int kind, double rturn, double speed, const mpb200_obstacles *o,
+                 const mpb200_space_desc *ss, int *blocks) {
+    SpaceDev S;
+    if (int rc = car_space(o, ss, &S)) return rc;
+    if (o->kind == 0) return gmt_launch(a, GmtCarEdge<0>{kind, rturn, speed, S, o->table.as<double>(), o->M}, blocks);
+    return gmt_launch(a, GmtCarEdge<1>{kind, rturn, speed, S, o->table.as<double>(), o->M}, blocks);
 }
 
 }  // namespace mpb

@@ -13,6 +13,7 @@
 #include "predicates.cuh"
 #include "philox.cuh"
 #include "scan.cuh"
+#include "gmt.cuh"
 #include <climits>
 #include <cstdlib>
 
@@ -601,6 +602,34 @@ int sample_free_device(const mpb200_obstacles *o, const mpb200_space_desc *ss, i
             return fail(MPB200_EARG, "no free state among %lld candidates: the free space is empty", (long long)cands);
     }
     *h_used = c.h_scalar[13];
+    return 0;
+}
+
+// lazy GMT*: step 4 runs motion_free (the segment test of segments_free_kernel) on the winning entry, on one lane
+template <int N, int DW, int KIND>
+struct GmtStraightEdge {
+    static constexpr bool kLazy = true;
+    SpaceDev S;
+    const double *T;
+    int M;
+    __device__ bool operator()(const GmtArgs &a, long long, int y, int x, GmtCtl *ctl) const {
+        double v[N], w[N];
+        gmt_endpoints<N>(a, y, x, v, w);
+        bool checked;
+        const bool ok = motion_free<N, DW, KIND>(S, T, M, v, w, &checked);
+        gmt_count_segments(ctl, checked ? 1 : 0);
+        return ok;
+    }
+};
+
+int gmt_lazy_straight(const GmtArgs &a, const mpb200_obstacles *o, const mpb200_space_desc *ss, int *blocks) {
+    SpaceDev S;
+    int dw = 0;
+    if (int rc = make_space(ss, a.d, &S, &dw)) return rc;
+    if (int rc = check_obstacles(o, dw)) return rc;
+#define CALL(N_, DW_, K_) return gmt_launch(a, GmtStraightEdge<N_, DW_, K_>{S, o->table.as<double>(), o->M}, blocks)
+    MPB_DISPATCH_DIMS(S.n, dw, o->kind, CALL);
+#undef CALL
     return 0;
 }
 

@@ -19,6 +19,7 @@
 #include "common.cuh"
 #include "predicates.cuh"
 #include "scan.cuh"
+#include "gmt.cuh"
 
 namespace mpb {
 
@@ -769,6 +770,39 @@ int lq_motions_free_device(const mpb200_lq *lq, double r, const double *dA, cons
     MPB_LQ_DISPATCH(lq->d, dw, o->kind, CALL);
 #undef CALL
     MPB_LAUNCHED();
+    return 0;
+}
+
+// lazy GMT*: step 4 runs lq_motion_free (the check of lq_edges_free_kernel) on the winning entry, on one lane
+template <int D, int DW, int KIND>
+struct GmtLqEdge {
+    static constexpr bool kLazy = true;
+    LqDev L;
+    double r;
+    SpaceDev S;
+    const double *T;
+    int M;
+    __device__ bool operator()(const GmtArgs &a, long long, int y, int x, GmtCtl *ctl) const {
+        double v[2 * D], w[2 * D];
+        gmt_endpoints<2 * D>(a, y, x, v, w);
+        int nchk = 0;
+        const bool ok = lq_motion_free<D, DW, KIND>(L, S, T, M, r, v, w, &nchk);
+        gmt_count_segments(ctl, nchk);
+        return ok;
+    }
+};
+
+int gmt_lazy_lq(const GmtArgs &a, const mpb200_lq *lq, double r, const mpb200_obstacles *o, const mpb200_space_desc *ss,
+                int *blocks) {
+    SpaceDev S;
+    int dw = 0;
+    if (int rc = make_space(ss, a.d, &S, &dw)) return rc;
+    if (a.d != 2 * lq->d) return fail(MPB200_EARG, "sample dimension %d != 2 x %d", a.d, lq->d);
+    if (o->kind == 1 && o->d != dw) return fail(MPB200_EARG, "box dimension %d != workspace dimension %d", o->d, dw);
+    const LqDev L = lq_dev(lq);
+#define CALL(D_, DW_, K_) return gmt_launch(a, GmtLqEdge<D_, DW_, K_>{L, r, S, o->table.as<double>(), o->M}, blocks)
+    MPB_LQ_DISPATCH(lq->d, dw, o->kind, CALL);
+#undef CALL
     return 0;
 }
 

@@ -277,14 +277,19 @@ def fmtstar(P, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, init_id
 
 
 def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1, init_idx=1, checkpts=True, seed=0,
-            k=None):
+            k=None, edge_checks="table"):
     """Group-marching FMT* (GMT*; Ichter, Schmerling & Pavone 2017) planned on the device -> (status, cost, elapsed)
 
     Sets the problem up exactly as fmtstar does (radius, steering, sample_free, goal mask), builds the tables and
     validity bits with the device-only calls and plans over them in one cooperative kernel (mpb200_gmt_plan): each
     iteration expands, all at once, every open vertex whose cost is within lam * r of the cheapest one.  No table
     crosses PCIe; the path, tree and costs come back.  At lam = 0 (and no two open vertices of equal cost) the tree,
-    path, cost and "collision_checks" equal fmtstar's.  Specification: include/mpb200.h, DESIGN.md section 10b."""
+    path, cost and "collision_checks" equal fmtstar's.  Specification: include/mpb200.h, DESIGN.md section 10b.
+
+    edge_checks = "table": every stored edge of the backward table is checked in one pass before planning and the
+    planner reads its bit.  edge_checks = "lazy": no edge pass; the planning kernel runs the motion check of the one
+    entry each candidate connects through (mpb200_gmt_plan_lazy), so only the motions the plan uses are checked.  Both
+    modes return the identical tree, path, cost and counters; lazy adds "segment_checks", the segment tests it ran."""
     from . import _lib
     import ctypes
 
@@ -295,6 +300,9 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
         raise ValueError("Connection type must be radial (:R) or k-nearest (:K)")
     if not lam >= 0:
         raise ValueError("lam must be a non-negative number")
+    if edge_checks not in ("table", "lazy"):
+        raise ValueError("edge_checks must be 'table' or 'lazy'")
+    lazy = edge_checks == "lazy"
     knn_mode = connections == "K"
     SS, CC = P.SS, P.CC
     if r > 0:
@@ -314,7 +322,7 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
     if not np.all(V[init_idx - 1] == P.init):
         raise RuntimeError("P.V[init_idx] must be the init state (fmt.jl:48-66)")
 
-    # ---- the same tables and bits as fmtstar(edge_checks="table"), left on the device -------------------
+    # ---- the same tables and bits as fmtstar(edge_checks="table"), left on the device (lazy: no bits) ---------
     lq = isinstance(SS.dist, LinearQuadratic)
     car = is_car_metric(SS.dist)
     if knn_mode and (lq or (car and not SS.dist.symmetric)):
@@ -322,25 +330,33 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
         setup_steering(SS, r)
         NN.r = r
         DF, DB = NN.table_mknnF, NN.table_knnB
-        (NN.car_edges_free if car else NN.lq_edges_free)(CC, SS, fetch=False, table=DB)
+        if not lazy:
+            (NN.car_edges_free if car else NN.lq_edges_free)(CC, SS, fetch=False, table=DB)
     elif knn_mode and car:
         r = NN.build_knn(k, r)
         setup_steering(SS, r)
         NN.r = r
         DF, DB = NN.table_mknn, NN.table_knn
-        NN.car_edges_free(CC, SS, fetch=False, table=DB)
+        if not lazy:
+            NN.car_edges_free(CC, SS, fetch=False, table=DB)
     elif knn_mode:
         NN.build_knn(k)
         DF, DB = NN.table_mknn, NN.table_knn
-        NN.edges_free(DB, CC, SS, fetch=False)
+        if not lazy:
+            NN.edges_free(DB, CC, SS, fetch=False)
     elif car and SS.dist.symmetric:
         NN.build_table(r)
         DF = DB = NN.table
-        NN.car_edges_free(CC, SS, fetch=False)
+        if not lazy:
+            NN.car_edges_free(CC, SS, fetch=False)
     elif car or lq:
         NN.build_tables(r)
         DF, DB = NN.tableF, NN.tableB
-        (NN.car_edges_free if car else NN.lq_edges_free)(CC, SS, fetch=False)
+        if not lazy:
+            (NN.car_edges_free if car else NN.lq_edges_free)(CC, SS, fetch=False)
+    elif lazy:
+        NN.build_table(r)
+        DF = DB = NN.table
     else:
         NN.build_table_checked(r, CC, SS)
         DF = DB = NN.table
@@ -361,8 +377,21 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
     C = np.empty(N, dtype=np.float64)
     path = np.empty(N, dtype=np.int64)
     lib = _lib.lib()
-    _lib.check(lib.mpb200_gmt_plan(NN.handle(), ctypes.byref(desc), ctypes.byref(res), _lib.ptr(path), N,
-                                   _lib.ptr(tree), _lib.ptr(C)))
+    if lazy:
+        if car:
+            m_ = NN.dist.m
+            edges = _lib.GmtEdges(_lib.GMT_EDGES_CAR, CC.handle(), None, 0.0, m_.kind, m_.r, m_.s)
+        elif lq:
+            edges = _lib.GmtEdges(_lib.GMT_EDGES_LQ, CC.handle(), NN.dist.handle(), NN.r, 0, 0.0, 0.0)
+        else:
+            edges = _lib.GmtEdges(_lib.GMT_EDGES_STRAIGHT, CC.handle(), None, 0.0, 0, 0.0, 0.0)
+        segment_checks = _lib.c_i64(0)
+        _lib.check(lib.mpb200_gmt_plan_lazy(NN.handle(), ctypes.byref(desc), ctypes.byref(edges), ctypes.byref(res),
+                                            ctypes.byref(segment_checks), _lib.ptr(path), N, _lib.ptr(tree),
+                                            _lib.ptr(C)))
+    else:
+        _lib.check(lib.mpb200_gmt_plan(NN.handle(), ctypes.byref(desc), ctypes.byref(res), _lib.ptr(path), N,
+                                       _lib.ptr(tree), _lib.ptr(C)))
     device_ms = lib.mpb200_last_ms_of(_lib.OP_PLAN, 0)
     solved = bool(res.solved)
     sol = [int(v) for v in path[:res.path_len]]
@@ -374,11 +403,13 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
     meta = {
         "radius_multiplier": rm, "collision_checks": checks, "num_samples": N, "cost": cost,
         "cumcost": [float(C[v - 1]) for v in sol], "planner": "GMTstar", "solved": solved, "tree": tree, "path": sol,
-        "r": r, "precomputed_edge_checks": int(lookups_before), "edge_checks": "table",
+        "r": r, "precomputed_edge_checks": int(lookups_before), "edge_checks": edge_checks,
         "connections": connections, "k": (k if knn_mode else None), "device_edge_batches": 0,
         "lambda": lam, "iterations": int(res.iterations), "expansions": int(res.expansions), "device_ms": device_ms,
         "costs": C, "checks": int(res.checks), "checks_in_bounds": int(res.checks_in_bounds),
         "grid_blocks": int(res.grid_blocks),
     }
+    if lazy:
+        meta["segment_checks"] = int(segment_checks.value)
     P.solution = MPSolution(P.status, cost, time.perf_counter() - t_start, meta)
     return P.status, P.solution.cost, P.solution.elapsed
