@@ -438,6 +438,29 @@ int mpb200_gmt_plan_lazy(const mpb200_samples *s, const mpb200_gmt_desc *desc, c
                          mpb200_gmt_result *res, int64_t *segment_checks, int64_t *path, int64_t path_cap,
                          int64_t *tree, double *costs);
 
+/* A batch of GMT* queries over one roadmap: nq independent plans over the same samples, the same fwd / bwd tables,
+ * point bits, checkpts setting and space, and the same edge test (edges == NULL: the edge bits of bwd, as
+ * mpb200_gmt_plan; else the motion check of edges, as mpb200_gmt_plan_lazy).  Query q has its own init, goal mask
+ * and width from descs[q].  Every output of query q (res[q] but grid_blocks, segment_checks[q], row q of paths,
+ * trees and costs) is byte-identical to what mpb200_gmt_plan / _lazy returns for descs[q] alone over the same tables,
+ * whatever the other queries of the batch, their order or the grid size.  grid_blocks is that of the one launch.
+ * The queries march in lockstep through one cooperative launch and share its grid-wide barriers; measured at C2 on one
+ * B200 (DESIGN.md section 10b), 16 queries cost 2.8x less than their single plans and 64 queries 4x less, and a batch
+ * lasts as long as its longest query.
+ * paths: nq x path_cap, row q = the path of query q, written only when its path_len <= path_cap (paths may be NULL
+ * when path_cap == 0); trees (int64) and costs (f64): nq x N each, row q = query q, may be NULL.
+ * Rejected with MPB200_EARG before any launch: everything mpb200_gmt_plan / _lazy rejects, for every query; nq < 1;
+ * NULL descs or res; descs whose fwd, bwd, checkpts or space differ from those of descs[0]; NULL paths with
+ * path_cap > 0.  MPB200_ENOMEM, without a launch, when the scratch of the batch cannot be reserved: per query
+ * MPB200_GMT_BATCH_BYTES_PER_QUERY(N, path_cap) bytes of device memory (C, A, status, four (query, vertex) lists, the
+ * path row, the goal mask, the control block).  One launch per call, timed under MPB200_OP_PLAN. */
+#define MPB200_GMT_BATCH_BYTES_PER_QUERY(N, path_cap) \
+    (52 * (int64_t)(N) + 8 * ((int64_t)(path_cap) < (int64_t)(N) ? (int64_t)(path_cap) : (int64_t)(N)) + \
+     8 * (((int64_t)(N) + 63) / 64) + 120)
+int mpb200_gmt_plan_batch(const mpb200_samples *s, const mpb200_gmt_desc *descs, int64_t nq,
+                          const mpb200_gmt_edges *edges, mpb200_gmt_result *res, int64_t *segment_checks,
+                          int64_t *paths, int64_t path_cap, int64_t *trees, double *costs);
+
 #ifdef __cplusplus
 }
 #endif

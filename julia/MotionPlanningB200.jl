@@ -422,4 +422,24 @@ function gmtstar_lazy_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::B
     r, path[1:r.path_len], tree, costs, segs[]
 end
 
+"""A batch of queries over one roadmap in one launch (mpb200_gmt_plan_batch): query q from sample inits[q] (1-based) to
+goals[q] at width ws[q], over the tables and bits of gmtstar_b200 (edges === nothing) or with the motion check of
+gmtstar_lazy_b200.  Each query's outputs equal that single call's for it.  Returns, per query, (result, path, tree,
+costs, segment tests run).  Declared only: Julia is not installed where this binding was written, so it has not been
+run."""
+function gmtstar_batch_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, inits::Vector{Int64}, goals::Vector{BitVector},
+                            ws::Vector{Float64}, sd::SpaceDesc, edges::Union{GmtEdgesC, Void} = nothing;
+                            checkpts = true)
+    nq = length(inits); N = length(goals[1])
+    descs = [GmtDescC(tF, tB, pointer(goals[q].chunks), inits[q], ws[q], Int32(checkpts),
+                      Base.unsafe_convert(Ptr{SpaceDescC}, sd.c)) for q in 1:nq]   # goals and sd stay rooted
+    res = Vector{GmtResultC}(nq); segs = zeros(Int64, nq)
+    paths = Matrix{Int64}(N, nq); trees = Matrix{Int64}(N, nq); costs = Matrix{Float64}(N, nq)   # column q = query q
+    check(ccall((:mpb200_gmt_plan_batch, LIB), Cint,
+                (Ptr{Void}, Ptr{GmtDescC}, Int64, Ptr{GmtEdgesC}, Ptr{GmtResultC}, Ptr{Int64}, Ptr{Int64}, Int64,
+                 Ptr{Int64}, Ptr{Float64}),
+                s.h, descs, nq, edges === nothing ? C_NULL : Ref(edges), res, segs, paths, N, trees, costs))
+    [(res[q], paths[1:res[q].path_len, q], trees[:, q], costs[:, q], segs[q]) for q in 1:nq]
+end
+
 end # module

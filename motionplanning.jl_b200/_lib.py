@@ -127,6 +127,8 @@ SIGNATURES = {
     "mpb200_gmt_plan": (ctypes.c_int, [c_vp, P(GmtDesc), P(GmtResult), c_vp, c_i64, c_vp, c_vp]),
     "mpb200_gmt_plan_lazy": (ctypes.c_int, [c_vp, P(GmtDesc), P(GmtEdges), P(GmtResult), P(c_i64), c_vp, c_i64, c_vp,
                                             c_vp]),
+    "mpb200_gmt_plan_batch": (ctypes.c_int, [c_vp, P(GmtDesc), c_i64, P(GmtEdges), P(GmtResult), c_vp, c_vp, c_i64,
+                                             c_vp, c_vp]),
 }
 
 _lib = None

@@ -276,51 +276,19 @@ def fmtstar(P, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, init_id
     return P.status, P.solution.cost, P.solution.elapsed
 
 
-def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1, init_idx=1, checkpts=True, seed=0,
-            k=None, edge_checks="table"):
-    """Group-marching FMT* (GMT*; Ichter, Schmerling & Pavone 2017) planned on the device -> (status, cost, elapsed)
-
-    Sets the problem up exactly as fmtstar does (radius, steering, sample_free, goal mask), builds the tables and
-    validity bits with the device-only calls and plans over them in one cooperative kernel (mpb200_gmt_plan): each
-    iteration expands, all at once, every open vertex whose cost is within lam * r of the cheapest one.  No table
-    crosses PCIe; the path, tree and costs come back.  At lam = 0 (and no two open vertices of equal cost) the tree,
-    path, cost and "collision_checks" equal fmtstar's.  Specification: include/mpb200.h, DESIGN.md section 10b.
-
-    edge_checks = "table": every stored edge of the backward table is checked in one pass before planning and the
-    planner reads its bit.  edge_checks = "lazy": no edge pass; the planning kernel runs the motion check of the one
-    entry each candidate connects through (mpb200_gmt_plan_lazy), so only the motions the plan uses are checked.  Both
-    modes return the identical tree, path, cost and counters; lazy adds "segment_checks", the segment tests it ran."""
-    from . import _lib
-    import ctypes
-
-    t_start = time.perf_counter()
-    N = len(P.V) if N is None else N
-    P.CC.count = 0
-    if connections not in ("R", "K"):
-        raise ValueError("Connection type must be radial (:R) or k-nearest (:K)")
-    if not lam >= 0:
-        raise ValueError("lam must be a non-negative number")
-    if edge_checks not in ("table", "lazy"):
-        raise ValueError("edge_checks must be 'table' or 'lazy'")
-    lazy = edge_checks == "lazy"
-    knn_mode = connections == "K"
+def _gmt_roadmap(P, N, rm, connections, r, ensure_goal_ct, checkpts, seed, k, lazy):
+    """The roadmap GMT* plans over, left on the device: sample_free up to N samples, the radius (fmt.jl:37-41) and
+    steering, the forward and backward tables of the connection type, the edge bits of the backward table (none when
+    lazy) and the point bits (checkpts).  -> dict(NN, DF, DB, r, k, lookups_before, lq, car, knn_mode)"""
     SS, CC = P.SS, P.CC
-    if r > 0:
-        setup_steering(SS, r)
-    if not states_free(P.init, CC, SS)[0]:
-        P.status = "failed"
-        P.solution = MPSolution(P.status, math.inf, time.perf_counter() - t_start, {})
-        return math.inf
+    knn_mode = connections == "K"
     free_volume_ub = sample_free(P, N - len(P.V), ensure_goal_ct=ensure_goal_ct, seed=seed) if N > len(P.V) else volume(SS)
     NN = P.V
-    V = NN.V
     if r == 0:
         r = fmt_radius(N, SS.dim, rm, free_volume_ub)
         setup_steering(SS, r)
     if k is None:
         k = min(int(math.ceil((2 * rm) ** SS.dim * (math.e / SS.dim) * math.log(N))), N - 1)
-    if not np.all(V[init_idx - 1] == P.init):
-        raise RuntimeError("P.V[init_idx] must be the init state (fmt.jl:48-66)")
 
     # ---- the same tables and bits as fmtstar(edge_checks="table"), left on the device (lazy: no bits) ---------
     lq = isinstance(SS.dist, LinearQuadratic)
@@ -364,27 +332,97 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
     CC.count = 0
     if checkpts:
         NN.points_free(CC, SS, fetch=False)
-    goal_chunks = np.zeros((N + 63) // 64 * 8, dtype=np.uint8)
-    packed = np.packbits(goal_mask(V, P.goal, SS), bitorder="little")
-    goal_chunks[:len(packed)] = packed
-    goal_chunks = goal_chunks.view(np.uint64)
+    return dict(NN=NN, DF=DF, DB=DB, r=r, k=k, lookups_before=lookups_before, lq=lq, car=car, knn_mode=knn_mode)
+
+
+def _gmt_edges(rm, CC):
+    """the lazy motion check of the roadmap's metric (mpb200_gmt_edges)"""
+    from . import _lib
+    NN = rm["NN"]
+    if rm["car"]:
+        m_ = NN.dist.m
+        return _lib.GmtEdges(_lib.GMT_EDGES_CAR, CC.handle(), None, 0.0, m_.kind, m_.r, m_.s)
+    if rm["lq"]:
+        return _lib.GmtEdges(_lib.GMT_EDGES_LQ, CC.handle(), NN.dist.handle(), NN.r, 0, 0.0, 0.0)
+    return _lib.GmtEdges(_lib.GMT_EDGES_STRAIGHT, CC.handle(), None, 0.0, 0, 0.0, 0.0)
+
+
+def _goal_chunks(V, goal, SS):
+    """the goal mask of V as host BitVector chunks (ceil(N/64) uint64 words)"""
+    chunks = np.zeros((len(V) + 63) // 64 * 8, dtype=np.uint8)
+    packed = np.packbits(goal_mask(V, goal, SS), bitorder="little")
+    chunks[:len(packed)] = packed
+    return chunks.view(np.uint64)
+
+
+def _gmt_check_args(connections, lams, edge_checks):
+    if connections not in ("R", "K"):
+        raise ValueError("Connection type must be radial (:R) or k-nearest (:K)")
+    if not all(lam >= 0 for lam in lams):
+        raise ValueError("lam must be a non-negative number")
+    if edge_checks not in ("table", "lazy"):
+        raise ValueError("edge_checks must be 'table' or 'lazy'")
+
+
+def _gmt_meta(rm, res, sol, C, tree, checks, lam, connections, edge_checks, device_ms, N, rmult):
+    return {
+        "radius_multiplier": rmult, "collision_checks": checks, "num_samples": N, "cost": float(res.cost),
+        "cumcost": None if C is None else [float(C[v - 1]) for v in sol], "planner": "GMTstar",
+        "solved": bool(res.solved), "tree": tree, "path": sol, "r": rm["r"],
+        "precomputed_edge_checks": int(rm["lookups_before"]), "edge_checks": edge_checks,
+        "connections": connections, "k": (rm["k"] if rm["knn_mode"] else None), "device_edge_batches": 0,
+        "lambda": lam, "iterations": int(res.iterations), "expansions": int(res.expansions), "device_ms": device_ms,
+        "costs": C, "checks": int(res.checks), "checks_in_bounds": int(res.checks_in_bounds),
+        "grid_blocks": int(res.grid_blocks),
+    }
+
+
+def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1, init_idx=1, checkpts=True, seed=0,
+            k=None, edge_checks="table"):
+    """Group-marching FMT* (GMT*; Ichter, Schmerling & Pavone 2017) planned on the device -> (status, cost, elapsed)
+
+    Sets the problem up exactly as fmtstar does (radius, steering, sample_free, goal mask), builds the tables and
+    validity bits with the device-only calls and plans over them in one cooperative kernel (mpb200_gmt_plan): each
+    iteration expands, all at once, every open vertex whose cost is within lam * r of the cheapest one.  No table
+    crosses PCIe; the path, tree and costs come back.  At lam = 0 (and no two open vertices of equal cost) the tree,
+    path, cost and "collision_checks" equal fmtstar's.  Specification: include/mpb200.h, DESIGN.md section 10b.
+
+    edge_checks = "table": every stored edge of the backward table is checked in one pass before planning and the
+    planner reads its bit.  edge_checks = "lazy": no edge pass; the planning kernel runs the motion check of the one
+    entry each candidate connects through (mpb200_gmt_plan_lazy), so only the motions the plan uses are checked.  Both
+    modes return the identical tree, path, cost and counters; lazy adds "segment_checks", the segment tests it ran."""
+    from . import _lib
+    import ctypes
+
+    t_start = time.perf_counter()
+    N = len(P.V) if N is None else N
+    P.CC.count = 0
+    _gmt_check_args(connections, [lam], edge_checks)
+    lazy = edge_checks == "lazy"
+    SS, CC = P.SS, P.CC
+    if r > 0:
+        setup_steering(SS, r)
+    if not states_free(P.init, CC, SS)[0]:
+        P.status = "failed"
+        P.solution = MPSolution(P.status, math.inf, time.perf_counter() - t_start, {})
+        return math.inf
+    rmap = _gmt_roadmap(P, N, rm, connections, r, ensure_goal_ct, checkpts, seed, k, lazy)
+    NN, DF, DB = rmap["NN"], rmap["DF"], rmap["DB"]
+    V = NN.V
+    if not np.all(V[init_idx - 1] == P.init):
+        raise RuntimeError("P.V[init_idx] must be the init state (fmt.jl:48-66)")
+    goal_chunks = _goal_chunks(V, P.goal, SS)
 
     space = SS.desc()
-    desc = _lib.GmtDesc(DF.h, DB.h, _lib.ptr(goal_chunks), init_idx, float(lam) * float(r), int(bool(checkpts)),
-                        ctypes.pointer(space))
+    desc = _lib.GmtDesc(DF.h, DB.h, _lib.ptr(goal_chunks), init_idx, float(lam) * float(rmap["r"]),
+                        int(bool(checkpts)), ctypes.pointer(space))
     res = _lib.GmtResult()
     tree = np.empty(N, dtype=np.int64)
     C = np.empty(N, dtype=np.float64)
     path = np.empty(N, dtype=np.int64)
     lib = _lib.lib()
     if lazy:
-        if car:
-            m_ = NN.dist.m
-            edges = _lib.GmtEdges(_lib.GMT_EDGES_CAR, CC.handle(), None, 0.0, m_.kind, m_.r, m_.s)
-        elif lq:
-            edges = _lib.GmtEdges(_lib.GMT_EDGES_LQ, CC.handle(), NN.dist.handle(), NN.r, 0, 0.0, 0.0)
-        else:
-            edges = _lib.GmtEdges(_lib.GMT_EDGES_STRAIGHT, CC.handle(), None, 0.0, 0, 0.0, 0.0)
+        edges = _gmt_edges(rmap, CC)
         segment_checks = _lib.c_i64(0)
         _lib.check(lib.mpb200_gmt_plan_lazy(NN.handle(), ctypes.byref(desc), ctypes.byref(edges), ctypes.byref(res),
                                             ctypes.byref(segment_checks), _lib.ptr(path), N, _lib.ptr(tree),
@@ -393,23 +431,87 @@ def gmtstar(P, N=None, rm=1.0, connections="R", r=0.0, lam=1.0, ensure_goal_ct=1
         _lib.check(lib.mpb200_gmt_plan(NN.handle(), ctypes.byref(desc), ctypes.byref(res), _lib.ptr(path), N,
                                        _lib.ptr(tree), _lib.ptr(C)))
     device_ms = lib.mpb200_last_ms_of(_lib.OP_PLAN, 0)
-    solved = bool(res.solved)
     sol = [int(v) for v in path[:res.path_len]]
     # fmtstar counts a Euclidean check only when y lies in the state bounds (the lazy checker's segment count)
-    checks = int(res.checks) if (lq or car) else int(res.checks_in_bounds)
-    P.status = "solved" if solved else "failed"
+    checks = int(res.checks) if (rmap["lq"] or rmap["car"]) else int(res.checks_in_bounds)
+    P.status = "solved" if res.solved else "failed"
     CC.count = checks
-    cost = float(res.cost)
-    meta = {
-        "radius_multiplier": rm, "collision_checks": checks, "num_samples": N, "cost": cost,
-        "cumcost": [float(C[v - 1]) for v in sol], "planner": "GMTstar", "solved": solved, "tree": tree, "path": sol,
-        "r": r, "precomputed_edge_checks": int(lookups_before), "edge_checks": edge_checks,
-        "connections": connections, "k": (k if knn_mode else None), "device_edge_batches": 0,
-        "lambda": lam, "iterations": int(res.iterations), "expansions": int(res.expansions), "device_ms": device_ms,
-        "costs": C, "checks": int(res.checks), "checks_in_bounds": int(res.checks_in_bounds),
-        "grid_blocks": int(res.grid_blocks),
-    }
+    meta = _gmt_meta(rmap, res, sol, C, tree, checks, lam, connections, edge_checks, device_ms, N, rm)
     if lazy:
         meta["segment_checks"] = int(segment_checks.value)
-    P.solution = MPSolution(P.status, cost, time.perf_counter() - t_start, meta)
+    P.solution = MPSolution(P.status, float(res.cost), time.perf_counter() - t_start, meta)
     return P.status, P.solution.cost, P.solution.elapsed
+
+
+def gmtstar_batch(P, inits, goals, lam=1.0, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, checkpts=True,
+                  seed=0, k=None, edge_checks="table", trees=True):
+    """A batch of GMT* queries over one roadmap -> [MPSolution], one per query
+
+    The roadmap is set up exactly as gmtstar sets it up (sample 1 = P.init, P.goal's goal samples, radius, steering,
+    tables, bits); then every query q, from sample inits[q] (1-based) to goals[q] (a goal object: its mask is goal_mask)
+    at width lam[q] * r (lam: a scalar or one value per query), is planned in one cooperative launch
+    (mpb200_gmt_plan_batch).  Each query's solution equals what gmtstar would return for it over the same roadmap;
+    a query whose init sample is not free is "failed" without a plan.  Metadata: gmtstar's keys plus "query" (its
+    position in the batch) and "batch_size"; "device_ms" is the time of the batch's kernel.  trees=False skips the
+    nq x N tree and cost copies ("tree", "costs" and "cumcost" are None)."""
+    from . import _lib
+    import ctypes
+
+    t_start = time.perf_counter()
+    inits = [int(i) for i in inits]
+    goals = list(goals)
+    nq = len(inits)
+    if nq == 0 or len(goals) != nq:
+        raise ValueError("inits and goals must be non-empty and of the same length")
+    lams = [float(x) for x in np.broadcast_to(np.asarray(lam, dtype=np.float64), (nq,))]
+    N = len(P.V) if N is None else N
+    P.CC.count = 0
+    _gmt_check_args(connections, lams, edge_checks)
+    if not all(1 <= i <= N for i in inits):
+        raise ValueError("inits must be sample indices 1..N")
+    lazy = edge_checks == "lazy"
+    SS, CC = P.SS, P.CC
+    if r > 0:
+        setup_steering(SS, r)
+    rmap = _gmt_roadmap(P, N, rm, connections, r, ensure_goal_ct, checkpts, seed, k, lazy)
+    NN, DF, DB = rmap["NN"], rmap["DF"], rmap["DB"]
+    V = NN.V
+    free = states_free(V[np.asarray(inits) - 1], CC, SS)      # fmt.jl:24-29, per query
+    planned = [q for q in range(nq) if free[q]]
+    n = len(planned)
+    space = SS.desc()
+    chunks = [_goal_chunks(V, goals[q], SS) for q in planned]
+    descs = (_lib.GmtDesc * max(n, 1))()
+    for j, q in enumerate(planned):
+        descs[j] = _lib.GmtDesc(DF.h, DB.h, _lib.ptr(chunks[j]), inits[q], lams[q] * float(rmap["r"]),
+                                int(bool(checkpts)), ctypes.pointer(space))
+    res = (_lib.GmtResult * max(n, 1))()
+    # a path can be N long, so each row holds N; np.empty only reserves address space and the library writes path_len
+    # entries of a row, so what becomes resident is the pages those paths touch (one 2 MB page a row with huge pages)
+    paths = np.empty((n, N), dtype=np.int64)
+    tree = np.empty((n, N), dtype=np.int64) if trees else None
+    C = np.empty((n, N), dtype=np.float64) if trees else None
+    segs = np.zeros(max(n, 1), dtype=np.int64)
+    lib = _lib.lib()
+    device_ms = 0.0
+    if n:
+        edges = ctypes.byref(_gmt_edges(rmap, CC)) if lazy else None
+        _lib.check(lib.mpb200_gmt_plan_batch(NN.handle(), descs, n, edges, res, _lib.ptr(segs) if lazy else None,
+                                             _lib.ptr(paths), N, _lib.ptr(tree), _lib.ptr(C)))
+        device_ms = lib.mpb200_last_ms_of(_lib.OP_PLAN, 0)
+    elapsed = time.perf_counter() - t_start
+    out = [MPSolution("failed", math.inf, elapsed, {"query": q, "batch_size": nq}) for q in range(nq)]
+    total_checks = 0
+    for j, q in enumerate(planned):
+        rq = res[j]
+        sol = [int(v) for v in paths[j, :rq.path_len]]
+        checks = int(rq.checks) if (rmap["lq"] or rmap["car"]) else int(rq.checks_in_bounds)
+        total_checks += checks
+        meta = _gmt_meta(rmap, rq, sol, None if C is None else C[j], None if tree is None else tree[j], checks,
+                         lams[q], connections, edge_checks, device_ms, N, rm)
+        if lazy:
+            meta["segment_checks"] = int(segs[j])
+        meta["query"], meta["batch_size"] = q, nq
+        out[q] = MPSolution("solved" if rq.solved else "failed", float(rq.cost), elapsed, meta)
+    CC.count = total_checks
+    return out
