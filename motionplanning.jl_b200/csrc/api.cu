@@ -181,9 +181,9 @@ int grid_inball_build(mpb200_samples *s, double r, mpb200_table *t);
 int brute_inball_build(mpb200_samples *s, double r, mpb200_table *t);
 
 int points_free_device(const double *dV, int64_t n, int d, const mpb200_obstacles *o, const mpb200_space_desc *ss,
-                       uint32_t *d_bits32, uint8_t *d_bytes, const int *order = nullptr);
-int edges_free_device(const double *dV, int d, const mpb200_table *t, const mpb200_obstacles *o,
-                      const mpb200_space_desc *ss, uint32_t *d_bits32, unsigned long long *d_checks);
+                       uint32_t *d_bits32, uint8_t *d_bytes, const mpb200_samples *cell_order = nullptr);
+int edges_free_device(const mpb200_samples *s, mpb200_table *t, const mpb200_obstacles *o,
+                      const mpb200_space_desc *ss, uint32_t *d_bits32, unsigned long long *d_counters);
 int segments_free_device(const double *dA, const double *dB, int64_t n, int d, const mpb200_obstacles *o,
                          const mpb200_space_desc *ss, uint8_t *d_out);
 
@@ -813,8 +813,7 @@ int mpb200_points_free(const mpb200_samples *s_, const mpb200_obstacles *o, cons
     phase_mark(0);
     MPB_CUDA(cudaMemsetAsync(s->point_bits.p, 0, sizeof(uint64_t) * (words + 1), st));
     // after a grid build the samples are visited in cell order: neighbouring lanes test neighbouring points
-    if (int rc = points_free_device(s->V.as<double>() + s->q0 * s->d, n, s->d, o, ss, s->point_bits.as<uint32_t>(), nullptr,
-                                    s->pt_order_valid ? s->pt_order.as<int>() : nullptr))
+    if (int rc = points_free_device(s->V.as<double>() + s->q0 * s->d, n, s->d, o, ss, s->point_bits.as<uint32_t>(), nullptr, s))
         return rc;
     s->point_bits_valid = s->q0 == 0 && s->q1 == s->N;
     phase_mark(1);
@@ -835,14 +834,15 @@ int mpb200_edges_free(const mpb200_samples *s, const mpb200_table *t_, const mpb
     Context &c = ctx();
     cudaStream_t st = c.stream;
     const size_t words = (size_t)ceil_div(t->nnz, 64);
-    if (int rc = t->edge_bits.reserve(sizeof(uint64_t) * (words + 1))) return rc;
+    // the bits, one spare word, then the pass's counters (segment tests run, columns left for the per-edge test):
+    // one memset clears them all
+    if (int rc = t->edge_bits.reserve(sizeof(uint64_t) * (words + 3))) return rc;
+    unsigned long long *d_counters = t->edge_bits.as<unsigned long long>() + words + 1;
     t->edge_bits_valid = false;
     phase_bank(MPB200_OP_EDGES);
     phase_mark(0);
-    MPB_CUDA(cudaMemsetAsync(t->edge_bits.p, 0, sizeof(uint64_t) * (words + 1), st));
-    MPB_CUDA(cudaMemsetAsync(c.d_scalar + 4, 0, sizeof(int64_t), st));
-    if (int rc = edges_free_device(s->V.as<double>(), s->d, t, o, ss, t->edge_bits.as<uint32_t>(),
-                                   reinterpret_cast<unsigned long long *>(c.d_scalar + 4)))
+    MPB_CUDA(cudaMemsetAsync(t->edge_bits.p, 0, sizeof(uint64_t) * (words + 3), st));
+    if (int rc = edges_free_device(s, t, o, ss, t->edge_bits.as<uint32_t>(), d_counters))
         return rc;
     t->edge_bits_valid = true;
     t->edge_bits_nnz = t->nnz;
@@ -851,7 +851,7 @@ int mpb200_edges_free(const mpb200_samples *s, const mpb200_table *t_, const mpb
     if (bitchunks || checks) {  // both NULL: asynchronous, the bits stay on the device
         if (bitchunks && words)
             MPB_CUDA(cudaMemcpyAsync(bitchunks, t->edge_bits.p, sizeof(uint64_t) * words, cudaMemcpyDeviceToHost, st));
-        MPB_CUDA(cudaMemcpyAsync(c.h_scalar + 4, c.d_scalar + 4, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
+        MPB_CUDA(cudaMemcpyAsync(c.h_scalar + 4, d_counters, sizeof(int64_t), cudaMemcpyDeviceToHost, st));
         MPB_CUDA(cudaStreamSynchronize(st));
         if (checks) *checks = c.h_scalar[4];
     }

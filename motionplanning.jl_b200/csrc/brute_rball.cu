@@ -468,6 +468,7 @@ static int brute_build(mpb200_samples *s, double r, mpb200_table *t) {
 }
 
 int brute_inball_build(mpb200_samples *s, double r, mpb200_table *t) {
+    s->pt_order_valid = false;  // sorted_pos and q_order are reused as FP32 scratch here
     switch (s->d) {
     case 4: return brute_build<4>(s, r, t);
     case 5: return brute_build<5>(s, r, t);

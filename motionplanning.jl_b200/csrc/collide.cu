@@ -6,9 +6,10 @@
 // batched over every stored entry of a neighbour table.  One lane per point / edge, the
 // obstacle table staged once per CTA into shared memory, results packed into Julia BitVector words
 // (bit k&63 of word k>>6 == bit k&31 of 32-bit word k>>5, little endian).  After a grid build the
-// points and the columns are visited in grid-cell order (the lanes of a warp then agree on which
-// obstacles they are near); classify_columns settles whole columns whose r-box is clear of every
-// obstacle (or inside one convex polygon) and only the rest reach the per-edge kernel.
+// points and the columns are visited in grid-cell order, read from the build's cell-ordered copy of
+// the samples (the lanes of a warp then agree on which obstacles they are near); classify_columns
+// settles whole columns whose r-box is clear of every obstacle (or inside one convex polygon) and only
+// the rest reach the per-edge kernel.
 #include "common.cuh"
 #include "predicates.cuh"
 #include "philox.cuh"
@@ -53,25 +54,52 @@ __device__ __forceinline__ bool motion_free(const SpaceDev &S, const double *T, 
     return box_segment_free<DW>(T, M, p, q);
 }
 
+// The grid build's cell-ordered copy of the sample set (grid_rball.cu): position t of the shard's cell-order
+// walk holds sample q0 + pt_order[t] at sorted_pos[pos], pos = q_order ? q_order[t] : t.
+struct CellOrder {
+    const double *pos;    // sorted_pos (N x d, AoS)
+    const int *q_order;   // shard: cell-order positions owned by the shard; NULL for the full range
+    const int *pt_order;  // sample (relative to q0) at walk position t
+};
+
 template <int N, int DW, int KIND>
 __global__ void __launch_bounds__(kThreads)
 points_free_kernel(const double *__restrict__ V, int64_t n, SpaceDev S, const double *__restrict__ g_table,
                    int table_words, int M, bool use_smem, uint32_t *__restrict__ bits32,
-                   uint8_t *__restrict__ bytes, const int *__restrict__ order) {
+                   uint8_t *__restrict__ bytes, CellOrder co) {
     extern __shared__ double s_table[];
     const double *T = stage_table(g_table, table_words, use_smem, s_table);
     const int64_t n_pad = (n + 31) & ~int64_t(31);
-    if (order) {
-        // points visited in grid-cell order (a permutation of 0 .. n-1): a warp's points are neighbours, so its
-        // lanes agree on which obstacles they are near; bits land in the pre-zeroed words with atomicOr
-        for (int64_t ti = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; ti < n; ti += (int64_t)gridDim.x * blockDim.x) {
-            const int64_t i = order[ti];
-            double v[N];
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    if (N <= 3 && co.pos) {  // grid builds cover d = 2, 3
+        // points visited in grid-cell order, read from the cell-ordered copy (coalesced): a warp's points are
+        // neighbours, so its lanes agree on which obstacles they are near; bits land in the pre-zeroed words with
+        // atomicOr.  The next point's loads are issued before the current point is tested.
+        int64_t ti = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+        double v[N];
+        int64_t i = 0;
+        if (ti < n) {
+            const int64_t pos = co.q_order ? co.q_order[ti] : ti;
 #pragma unroll
-            for (int k = 0; k < N; ++k) v[k] = V[i * N + k];
+            for (int k = 0; k < N; ++k) v[k] = co.pos[pos * N + k];
+            i = co.pt_order[ti];
+        }
+        while (ti < n) {
+            const int64_t tn = ti + stride;
+            double vn[N];
+            int64_t in = 0;
+            if (tn < n) {
+                const int64_t pos = co.q_order ? co.q_order[tn] : tn;
+#pragma unroll
+                for (int k = 0; k < N; ++k) vn[k] = co.pos[pos * N + k];
+                in = co.pt_order[tn];
+            }
             const bool ok = state_free<N, DW, KIND>(S, T, M, v);
             if (bits32 && ok) atomicOr(&bits32[i >> 5], 1u << (i & 31));
             if (bytes) bytes[i] = ok ? 1 : 0;
+            ti = tn; i = in;
+#pragma unroll
+            for (int k = 0; k < N; ++k) v[k] = vn[k];
         }
         return;
     }
@@ -89,83 +117,71 @@ points_free_kernel(const double *__restrict__ V, int64_t n, SpaceDev S, const do
     }
 }
 
-// One warp per column x of the table: the 32 lanes hold stored entries (row y -> column x) of
-// that column, i.e. edges sharing the endpoint V[x] (coherent control flow, no per-edge search
-// for the column).  The next column's colptr pair is prefetched while the current one is
-// processed.  Validity bits go to the (pre-zeroed) BitVector words with at most two atomicOr
-// per 32 edges; the per-CTA check counter is reduced before one atomicAdd.
-template <int N, int DW, int KIND>
-__global__ void __launch_bounds__(kThreads, (DW <= 3) ? 3 : 1)
-edges_free_kernel(const double *__restrict__ V, const int64_t *__restrict__ colptr,
-                  const int64_t *__restrict__ rowval, int64_t ncols, int64_t col0, int64_t nnz, SpaceDev S,
-                  const double *__restrict__ g_table, int table_words, int M, bool use_smem,
-                  uint32_t *__restrict__ bits32, unsigned long long *__restrict__ checks,
-                  const int *__restrict__ col_list, int64_t n_items, const unsigned long long *__restrict__ n_items_dev) {
-    extern __shared__ double s_table[];
-    const double *T = stage_table(g_table, table_words, use_smem, s_table);
-    if (n_items_dev) n_items = (int64_t)*n_items_dev;  // list length produced by classify_columns
-    const int lane = threadIdx.x & 31;
-    const int64_t gwarp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
-    unsigned long long my_checks = 0;
-    // 2-D compound: decode the table header once and keep this lane's cull box in registers
+// The 2-D compound's cull boxes for warp_line_colliding_2d: lane s keeps box s in registers (S <= 32).
+struct LaneCull {
+    double xl, xh, yl, yh;
+};
+template <int KIND>
+__device__ __forceinline__ LaneCull lane_cull(const Obs2 &O) {
     const double inf = __longlong_as_double(0x7ff0000000000000LL);
-    double cull_xl = inf, cull_xh = -inf, cull_yl = inf, cull_yh = -inf;
-    Obs2 O(KIND == 0 ? T : nullptr, KIND == 0);
+    LaneCull c{inf, -inf, inf, -inf};
+    const int lane = threadIdx.x & 31;
     if (KIND == 0 && lane < O.S && O.S <= 32) {
         const double *cb = O.cull_box(lane);
-        cull_xl = cb[0]; cull_xh = cb[1]; cull_yl = cb[2]; cull_yh = cb[3];
+        c = LaneCull{cb[0], cb[1], cb[2], cb[3]};
     }
-    // work item i -> column (optionally through a column list: the big-column leftovers of the fused build)
-    int64_t it = gwarp, c = 0, beg = 0, end = 0;
-    if (it < n_items) { c = col_list ? col_list[it] : it; beg = colptr[c] - 1; end = colptr[c + 1] - 1; }
-    while (it < n_items) {
-        const int64_t itn = it + nwarps;
-        int64_t cn = 0, begn = 0, endn = 0;
-        if (itn < n_items) { cn = col_list ? col_list[itn] : itn; begn = colptr[cn] - 1; endn = colptr[cn + 1] - 1; }  // prefetch
-        if (beg < end) {
-            double b[N], q[DW];
+    return c;
+}
+
+// Per-edge test of the stored entries [beg, end) of one column (row y -> column x), i.e. edges sharing the
+// endpoint x whose workspace image is q: the 32 lanes take 32 entries at a time (coherent control flow, no
+// per-edge search for the column).  y0 is rowval[beg + lane] - 1 where beg + lane < end, loaded by the caller
+// ahead of time.  Validity bits go to the (pre-zeroed) BitVector words with at most two atomicOr per 32 edges.
+template <int N, int DW, int KIND>
+__device__ __forceinline__ void column_edges(const SpaceDev &S, const double *T, int M, const Obs2 &O,
+                                             const LaneCull &cl, const double *__restrict__ V,
+                                             const int64_t *__restrict__ rowval, int64_t beg, int64_t end,
+                                             const double *q, int64_t y0, uint32_t *__restrict__ bits32,
+                                             unsigned long long &my_checks) {
+    const int lane = threadIdx.x & 31;
+    for (int64_t e0 = beg; e0 < end; e0 += 32) {
+        const int64_t e = e0 + lane;
+        bool run = false;
+        double a[N], p[DW];
 #pragma unroll
-            for (int k = 0; k < N; ++k) b[k] = V[(col0 + c) * N + k];
-            state2workspace<N, DW>(S, b, q);  // the last waypoint is never bounds-checked (Q4)
-            for (int64_t e0 = beg; e0 < end; e0 += 32) {
-                const int64_t e = e0 + lane;
-                bool run = false;
-                double a[N], p[DW];
+        for (int k = 0; k < N; ++k) a[k] = 0.0;
+        if (e < end) {
+            const int64_t y = e0 == beg ? y0 : rowval[e] - 1;
 #pragma unroll
-                for (int k = 0; k < N; ++k) a[k] = 0.0;
-                if (e < end) {
-                    const int64_t y = rowval[e] - 1;
-#pragma unroll
-                    for (int k = 0; k < N; ++k) a[k] = V[y * N + k];
-                    run = in_state_space<N>(S, a);  // statespaces.jl:155: in_state_space(wps[1]) && segment test
-                }
-                state2workspace<N, DW>(S, a, p);
-                my_checks += run ? 1 : 0;
-                // warp-collective: every lane must make the call (no short-circuit on `run`)
-                bool seg_free;
-                if (KIND == 0)
-                    seg_free = !warp_line_colliding_2d(O, cull_xl, cull_xh, cull_yl, cull_yh, p[0], p[DW > 1 ? 1 : 0], q[0],
-                                                       q[DW > 1 ? 1 : 0], run);
-                else
-                    seg_free = warp_box_segment_free<DW>(T, M, p, q, run);
-                const bool ok = run && seg_free;
-                const unsigned m = __ballot_sync(0xffffffffu, ok);
-                if (lane == 0 && m) {
-                    const int sh = (int)(e0 & 31);
-                    const int64_t wi = e0 >> 5;
-                    atomicOr(&bits32[wi], m << sh);
-                    if (sh && (m >> (32 - sh))) atomicOr(&bits32[wi + 1], m >> (32 - sh));
-                }
-            }
+            for (int k = 0; k < N; ++k) a[k] = V[y * N + k];
+            run = in_state_space<N>(S, a);  // statespaces.jl:155: in_state_space(wps[1]) && segment test
         }
-        it = itn; c = cn; beg = begn; end = endn;
+        state2workspace<N, DW>(S, a, p);
+        my_checks += run ? 1 : 0;
+        // warp-collective: every lane must make the call (no short-circuit on `run`)
+        bool seg_free;
+        if (KIND == 0)
+            seg_free = !warp_line_colliding_2d(O, cl.xl, cl.xh, cl.yl, cl.yh, p[0], p[DW > 1 ? 1 : 0], q[0],
+                                               q[DW > 1 ? 1 : 0], run);
+        else
+            seg_free = warp_box_segment_free<DW>(T, M, p, q, run);
+        const bool ok = run && seg_free;
+        const unsigned m = __ballot_sync(0xffffffffu, ok);
+        if (lane == 0 && m) {
+            const int sh = (int)(e0 & 31);
+            const int64_t wi = e0 >> 5;
+            atomicOr(&bits32[wi], m << sh);
+            if (sh && (m >> (32 - sh))) atomicOr(&bits32[wi + 1], m >> (32 - sh));
+        }
     }
-    // per-CTA reduction of the CC.count increment
+}
+
+// per-CTA reduction of the CC.count increment, then one atomicAdd
+__device__ __forceinline__ void add_checks(unsigned long long my_checks, unsigned long long *checks) {
     __shared__ unsigned long long s_checks[kThreads / 32];
 #pragma unroll
     for (int o = 16; o; o >>= 1) my_checks += __shfl_xor_sync(0xffffffffu, my_checks, o);
-    if (lane == 0) s_checks[threadIdx.x >> 5] = my_checks;
+    if ((threadIdx.x & 31) == 0) s_checks[threadIdx.x >> 5] = my_checks;
     __syncthreads();
     if (threadIdx.x == 0) {
         unsigned long long t = 0;
@@ -174,111 +190,161 @@ edges_free_kernel(const double *__restrict__ V, const int64_t *__restrict__ colp
     }
 }
 
-// One thread per column of a Euclidean r-ball table (state == workspace): every stored neighbour
-// lies within r of the column point x, so all edges of the column live inside the box x +- r.  If
-// that box is inside the state bounds and overlaps no obstacle's cull box, every edge passes
-// in_state_space and is rejected by every obstacle's own AABB gate: the whole column is free.  Its
-// validity bits are set here (<= 3 atomicOr), `checks` advances by the column length, and the
-// column never reaches the per-edge kernel.  Anything else is appended to `list`.
+// One warp per column of the table (any table, any state-to-workspace map), in column order -- or, after
+// classify_columns, per column of its list (length on the device).  The next column's colptr pair is prefetched while
+// the current one is processed.
+template <int N, int DW, int KIND>
+__global__ void __launch_bounds__(kThreads, (DW <= 3) ? 3 : 1)
+edges_free_kernel(const double *__restrict__ V, const int64_t *__restrict__ colptr,
+                  const int64_t *__restrict__ rowval, int64_t ncols, int64_t col0, SpaceDev S,
+                  const double *__restrict__ g_table, int table_words, int M, bool use_smem,
+                  uint32_t *__restrict__ bits32, unsigned long long *__restrict__ checks,
+                  const int *__restrict__ col_list, const unsigned long long *__restrict__ n_list) {
+    extern __shared__ double s_table[];
+    const double *T = stage_table(g_table, table_words, use_smem, s_table);
+    const int lane = threadIdx.x & 31;
+    const int64_t n_items = col_list ? (int64_t)*n_list : ncols;
+    const int64_t gwarp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    unsigned long long my_checks = 0;
+    Obs2 O(KIND == 0 ? T : nullptr, KIND == 0);
+    const LaneCull cl = lane_cull<KIND>(O);
+    int64_t it = gwarp, c = 0, beg = 0, end = 0;
+    if (it < n_items) { c = col_list ? col_list[it] : it; beg = colptr[c] - 1; end = colptr[c + 1] - 1; }
+    while (it < n_items) {
+        const int64_t itn = it + nwarps;
+        int64_t cn = 0, begn = 0, endn = 0;
+        if (itn < n_items) { cn = col_list ? col_list[itn] : itn; begn = colptr[cn] - 1; endn = colptr[cn + 1] - 1; }  // prefetch
+        if (beg < end) {
+            const int64_t y0 = beg + lane < end ? rowval[beg + lane] - 1 : 0;
+            double b[N], q[DW];
+#pragma unroll
+            for (int k = 0; k < N; ++k) b[k] = V[(col0 + c) * N + k];
+            state2workspace<N, DW>(S, b, q);  // the last waypoint is never bounds-checked (Q4)
+            column_edges<N, DW, KIND>(S, T, M, O, cl, V, rowval, beg, end, q, y0, bits32, my_checks);
+        }
+        it = itn; c = cn; beg = begn; end = endn;
+    }
+    add_checks(my_checks, checks);
+}
+
+// Column classes of a Euclidean r-ball table (state == workspace): every stored neighbour lies within r of the
+// column point x, so all edges of the column live inside the box x +- r.
+enum : int { kColFree = 0, kColColliding = 1, kColEdges = 2 };
+// If the box is inside the state bounds and overlaps no obstacle's cull box, every edge passes in_state_space
+// and is rejected by every obstacle's own AABB gate: the whole column is free.  If (2-D) the box sits inside one
+// convex polygon, every edge collides.  Anything else needs the per-edge test.
+template <int DW, int KIND>
+__device__ __forceinline__ int classify_column(const SpaceDev &S, const double *T, int M, double r, const double *x) {
+    double lo[DW], hi[DW];
+    bool trivial = true;
+#pragma unroll
+    for (int i = 0; i < DW; ++i) {
+        const double pad = r * (1.0 + 1e-9) + 4.5e-16 * fabs(x[i]);  // covers every rounding in x +- r
+        lo[i] = x[i] - pad; hi[i] = x[i] + pad;
+        trivial = trivial && (S.lo[i] <= lo[i] && hi[i] <= S.hi[i]);
+    }
+    if (!trivial) return kColEdges;
+    if (KIND == 0) {
+        Obs2 O(T);
+        const double ylo = lo[DW > 1 ? 1 : 0], yhi = hi[DW > 1 ? 1 : 0];
+        for (int s = 0; s < O.S; ++s) {
+            const double *cb = O.cull_box(s);
+            if (!(overlapping(lo[0], hi[0], cb[0], cb[1]) && overlapping(ylo, yhi, cb[2], cb[3]))) continue;
+            trivial = false;
+            // Both endpoints of every edge of the column lie in the box; if the box is inside
+            // polygon s by a margin far above rounding, no axis of the SAT test separates
+            // (SAT2D.jl:172-176), so every edge collides -- given the gate chain passes, which
+            // holds for consistent gates because they contain the polygon's AABB.
+            if (O.kind(s) == 1 && O.consistent()) {
+                const double *P = O.data(s);
+                const int K = O.K(s);
+                const double *nrm = P + 4 + 2 * K, *ext = P + 4 + 4 * K;
+                const double m = 1e-9 * (1.0 + fabs(lo[0]) + fabs(hi[0]) + fabs(ylo) + fabs(yhi));
+                bool inside = true;
+                for (int i = 0; i < K && inside; ++i) {
+                    const double n1 = nrm[2 * i], n2 = nrm[2 * i + 1];
+                    const double dmax = fmax(lo[0] * n1, hi[0] * n1) + fmax(ylo * n2, yhi * n2);
+                    inside = dmax <= ext[2 * i + 1] - m;  // support of the box along the outward normal
+                }
+                if (inside) return kColColliding;
+            }
+        }
+        return trivial ? kColFree : kColEdges;
+    }
+    const double *bl = T, *bh = T + (size_t)M * DW;
+    for (int k = 0; k < M; ++k) {
+        bool sep = false;
+#pragma unroll
+        for (int i = 0; i < DW; ++i) sep = sep || (bh[k * DW + i] < lo[i] || bl[k * DW + i] > hi[i]);
+        if (!sep) return kColEdges;
+    }
+    return kColFree;
+}
+
+// One lane per column of a Euclidean r-ball table with an identity state-to-workspace map, in grid-cell order when
+// the table has one (the lanes of a warp then look at neighbouring points and take the same branches), from a grid
+// of resident CTAs.  The column point comes from the grid build's cell-ordered copy when it describes this table
+// (a coalesced read), else from V.  The next column's id, colptr pair and point are loaded before the current one
+// is classified.  Free columns get their bits here (<= 3 atomicOr) and colliding ones nothing; both advance
+// `checks` by the column length.  The rest are appended to `list` (one atomicAdd per warp) for edges_free_kernel.
+// counters: [0] segment tests run (CC.count), [1] list length -- zeroed before the launch.
 template <int DW, int KIND>
 __global__ void __launch_bounds__(kThreads)
 classify_columns(const double *__restrict__ V, const int64_t *__restrict__ colptr, int64_t ncols, int64_t col0,
                  double r, SpaceDev S, const double *__restrict__ g_table, int table_words, int M, bool use_smem,
-                 unsigned long long *__restrict__ bits64, unsigned long long *__restrict__ checks,
-                 int *__restrict__ list, unsigned long long *__restrict__ n_list, const int *__restrict__ order) {
+                 const int *__restrict__ col_order, CellOrder co, uint32_t *__restrict__ bits32,
+                 unsigned long long *__restrict__ counters, int *__restrict__ list) {
     extern __shared__ double s_table[];
     const double *T = stage_table(g_table, table_words, use_smem, s_table);
     const int lane = threadIdx.x & 31;
     unsigned long long my_checks = 0;
-    const int64_t n_pad = (ncols + 31) & ~int64_t(31);
-    // `order` (optional) lists the columns in grid-cell order: the lanes of a warp then look at neighbouring
-    // points, take the same branches below, and the flagged list comes out spatially coherent too
-    for (int64_t ti = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; ti < n_pad; ti += (int64_t)gridDim.x * blockDim.x) {
-        bool flagged = false;
-        int64_t c = ti;
-        if (ti < ncols) {
-            if (order) c = order[ti];
-            const int64_t beg = colptr[c] - 1, end = colptr[c + 1] - 1;
-            if (beg < end) {
-                double lo[DW], hi[DW];
-                bool trivial = true;
+    unsigned long long *bits64 = reinterpret_cast<unsigned long long *>(bits32);
+    const double *P = co.pos ? co.pos : V;
+    const int64_t n_pad = (ncols + 31) & ~int64_t(31);  // whole warps: the ballot below needs every lane
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    // walk position t -> column c, its stored entries [beg, end) and its point
+    auto load = [&](int64_t t, int64_t &c, int64_t &beg, int64_t &end, double *x) {
+        beg = end = 0;
+        if (t < ncols) {
+            c = col_order ? col_order[t] : t;
+            beg = colptr[c] - 1; end = colptr[c + 1] - 1;
+            const int64_t xo = (co.pos ? (co.q_order ? co.q_order[t] : t) : col0 + c) * DW;
 #pragma unroll
-                for (int i = 0; i < DW; ++i) {
-                    const double x = V[(col0 + c) * DW + i];
-                    const double pad = r * (1.0 + 1e-9) + 4.5e-16 * fabs(x);  // covers every rounding in x +- r
-                    lo[i] = x - pad; hi[i] = x + pad;
-                    trivial = trivial && (S.lo[i] <= lo[i] && hi[i] <= S.hi[i]);
-                }
-                bool all_colliding = false;  // 2-D only: the whole r-box sits inside one convex polygon
-                if (trivial) {
-                    if (KIND == 0) {
-                        Obs2 O(T);
-                        const double ylo = lo[DW > 1 ? 1 : 0], yhi = hi[DW > 1 ? 1 : 0];
-                        for (int s = 0; s < O.S; ++s) {
-                            const double *cb = O.cull_box(s);
-                            if (!(overlapping(lo[0], hi[0], cb[0], cb[1]) && overlapping(ylo, yhi, cb[2], cb[3]))) continue;
-                            trivial = false;
-                            // Both endpoints of every edge of the column lie in the box; if the box is inside
-                            // polygon s by a margin far above rounding, no axis of the SAT test separates
-                            // (SAT2D.jl:172-176), so every edge collides -- given the gate chain passes, which
-                            // holds for consistent gates because they contain the polygon's AABB.
-                            if (O.kind(s) == 1 && O.consistent()) {
-                                const double *P = O.data(s);
-                                const int K = O.K(s);
-                                const double *nrm = P + 4 + 2 * K, *ext = P + 4 + 4 * K;
-                                const double m = 1e-9 * (1.0 + fabs(lo[0]) + fabs(hi[0]) + fabs(ylo) + fabs(yhi));
-                                bool inside = true;
-                                for (int i = 0; i < K && inside; ++i) {
-                                    const double n1 = nrm[2 * i], n2 = nrm[2 * i + 1];
-                                    const double dmax = fmax(lo[0] * n1, hi[0] * n1) + fmax(ylo * n2, yhi * n2);
-                                    inside = dmax <= ext[2 * i + 1] - m;  // support of the box along the outward normal
-                                }
-                                if (inside) { all_colliding = true; break; }
-                            }
-                        }
-                    } else {
-                        const double *bl = T, *bh = T + (size_t)M * DW;
-                        for (int k = 0; k < M && trivial; ++k) {
-                            bool sep = false;
-#pragma unroll
-                            for (int i = 0; i < DW; ++i) sep = sep || (bh[k * DW + i] < lo[i] || bl[k * DW + i] > hi[i]);
-                            if (!sep) trivial = false;
-                        }
-                    }
-                }
-                if (all_colliding) {
-                    my_checks += (unsigned long long)(end - beg);  // every segment test runs and fails: bits stay 0
-                } else if (trivial) {
-                    my_checks += (unsigned long long)(end - beg);
-                    for (int64_t w = beg >> 6; w <= (end - 1) >> 6; ++w) {
-                        const int64_t b0 = w << 6;
-                        const int from = (int)(beg > b0 ? beg - b0 : 0), to = (int)(end < b0 + 64 ? end - b0 : 64);
-                        const unsigned long long m = (to - from == 64) ? ~0ULL : (((1ULL << (to - from)) - 1ULL) << from);
-                        atomicOr(&bits64[w], m);
-                    }
-                } else {
-                    flagged = true;
-                }
+            for (int i = 0; i < DW; ++i) x[i] = P[xo + i];
+        }
+    };
+    int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    int64_t c = 0, beg, end;
+    double x[DW];
+    load(t, c, beg, end, x);
+    while (t < n_pad) {
+        const int64_t tn = t + stride;
+        int64_t cn = 0, begn, endn;
+        double xn[DW];
+        load(tn, cn, begn, endn, xn);  // prefetch
+        const int cls = beg < end ? classify_column<DW, KIND>(S, T, M, r, x) : kColFree;
+        if (cls != kColEdges) my_checks += (unsigned long long)(end - beg);  // colliding: every test runs and fails
+        if (cls == kColFree) {
+            for (int64_t w = beg >> 6; beg < end && w <= (end - 1) >> 6; ++w) {
+                const int64_t b0 = w << 6;
+                const int from = (int)(beg > b0 ? beg - b0 : 0), to = (int)(end < b0 + 64 ? end - b0 : 64);
+                const unsigned long long m = (to - from == 64) ? ~0ULL : (((1ULL << (to - from)) - 1ULL) << from);
+                atomicOr(&bits64[w], m);
             }
         }
-        const unsigned fm = __ballot_sync(0xffffffffu, flagged);
+        const unsigned fm = __ballot_sync(0xffffffffu, cls == kColEdges);
         if (fm) {
-            unsigned long long basei = 0;
-            if (lane == 0) basei = atomicAdd(n_list, (unsigned long long)__popc(fm));
-            basei = __shfl_sync(0xffffffffu, basei, 0);
-            if (flagged) list[basei + __popc(fm & ((1u << lane) - 1u))] = (int)c;
+            unsigned long long base = 0;
+            if (lane == 0) base = atomicAdd(&counters[1], (unsigned long long)__popc(fm));
+            base = __shfl_sync(0xffffffffu, base, 0);
+            if (cls == kColEdges) list[base + __popc(fm & ((1u << lane) - 1u))] = (int)c;
         }
-    }
-    __shared__ unsigned long long s_checks[kThreads / 32];
+        t = tn; c = cn; beg = begn; end = endn;
 #pragma unroll
-    for (int o = 16; o; o >>= 1) my_checks += __shfl_xor_sync(0xffffffffu, my_checks, o);
-    if (lane == 0) s_checks[threadIdx.x >> 5] = my_checks;
-    __syncthreads();
-    if (threadIdx.x == 0) {
-        unsigned long long tt = 0;
-        for (int w = 0; w < kThreads / 32; ++w) tt += s_checks[w];
-        if (tt) atomicAdd(checks, tt);
+        for (int i = 0; i < DW; ++i) x[i] = xn[i];
     }
+    add_checks(my_checks, &counters[0]);
 }
 
 template <int N, int DW, int KIND>
@@ -374,6 +440,24 @@ static int prep_kernel(K kernel, size_t smem) {
     return 0;
 }
 
+// Grid of the validity kernels (K6, K7/K8): every thread loops over its items, so one wave of resident CTAs
+// does the work -- as many as the occupancy calculator fits on the GPU at this shared-memory size, fewer when
+// there are fewer than that many CTAs' worth of items.  Call after prep_kernel (it sets the shared-memory limit).
+template <class K>
+static int resident_grid(K kernel, size_t smem, int64_t items, unsigned *grid) {
+    static size_t cached_smem = ~size_t(0);  // per kernel: the occupancy query is a host call per launch otherwise
+    static int per_sm = 0;
+    if (smem != cached_smem) {
+        MPB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem));
+        if (per_sm < 1) per_sm = 1;
+        cached_smem = smem;
+    }
+    const int64_t cap = (int64_t)per_sm * ctx().sm_count;
+    const int64_t blocks = ceil_div(items > 0 ? items : 1, kThreads);
+    *grid = (unsigned)(blocks < cap ? blocks : cap);
+    return 0;
+}
+
 int make_space(const mpb200_space_desc *ss, int d_state, SpaceDev *out, int *dw) {
     MPB_CHECK_ARG(ss != nullptr, "space descriptor is NULL");
     MPB_CHECK_ARG(ss->n == d_state, "space dimension does not match the sample dimension");
@@ -440,19 +524,29 @@ static int check_obstacles(const mpb200_obstacles *o, int dw) {
     return 0;
 }
 
+// The cell-ordered copy of the last grid build, while it describes the samples' current shard (cleared by every
+// other builder that reuses those buffers and by a change of the query range).
+static CellOrder cell_order(const mpb200_samples *s) {
+    if (!s || !s->pt_order_valid) return CellOrder{nullptr, nullptr, nullptr};
+    return CellOrder{s->sorted_pos.as<double>(), (s->q1 - s->q0 != s->N) ? s->q_order.as<int>() : nullptr,
+                     s->pt_order.as<int>()};
+}
+
 int points_free_device(const double *dV, int64_t n, int d, const mpb200_obstacles *o, const mpb200_space_desc *ss,
-                       uint32_t *d_bits32, uint8_t *d_bytes, const int *order) {
+                       uint32_t *d_bits32, uint8_t *d_bytes, const mpb200_samples *cs) {
     SpaceDev S;
     int dw = 0;
     if (int rc = make_space(ss, d, &S, &dw)) return rc;
     if (int rc = check_obstacles(o, dw)) return rc;
     LaunchCfg L = make_cfg(o, n);
+    const CellOrder co = cell_order(cs);
     cudaStream_t st = ctx().stream;
 #define CALL(N_, DW_, K_)                                                                              \
     do {                                                                                               \
         if (int rc = prep_kernel(points_free_kernel<N_, DW_, K_>, L.smem)) return rc;                  \
+        if (int rc = resident_grid(points_free_kernel<N_, DW_, K_>, L.smem, n, &L.grid)) return rc;    \
         points_free_kernel<N_, DW_, K_><<<L.grid, kThreads, L.smem, st>>>(dV, n, S, L.table, L.words, L.M, \
-                                                                          L.use_smem, d_bits32, d_bytes, order); \
+                                                                          L.use_smem, d_bits32, d_bytes, co); \
     } while (0)
     MPB_DISPATCH_DIMS(S.n, dw, o->kind, CALL);
 #undef CALL
@@ -460,69 +554,61 @@ int points_free_device(const double *dV, int64_t n, int d, const mpb200_obstacle
     return 0;
 }
 
-int edges_free_device_cols(const double *dV, int d, const mpb200_table *t, const mpb200_obstacles *o,
-                           const SpaceDev &S, uint32_t *d_bits32, unsigned long long *d_checks, const int *col_list,
-                           int64_t n_list, const unsigned long long *n_list_dev = nullptr);
-
-int edges_free_device(const double *dV, int d, const mpb200_table *t, const mpb200_obstacles *o,
-                      const mpb200_space_desc *ss, uint32_t *d_bits32, unsigned long long *d_checks) {
+int edges_free_device(const mpb200_samples *s, mpb200_table *t, const mpb200_obstacles *o,
+                      const mpb200_space_desc *ss, uint32_t *d_bits32, unsigned long long *d_counters) {
     SpaceDev S;
     int dw = 0;
-    if (int rc = make_space(ss, d, &S, &dw)) return rc;
+    if (int rc = make_space(ss, s->d, &S, &dw)) return rc;
     if (int rc = check_obstacles(o, dw)) return rc;
-    static const bool no_classify = getenv("MPB200_NO_CLASSIFY") != nullptr;
-    if (!(t->euclid && S.s2w_kind == 0 && t->ncols > 0 && t->ncols < INT_MAX) || no_classify)
-        return edges_free_device_cols(dV, d, t, o, S, d_bits32, d_checks, nullptr, t->ncols);
-    // classify pass: trivially-free columns are finished here, the rest go through the per-edge kernel
-    mpb200_table *tm = const_cast<mpb200_table *>(t);
-    if (int rc = tm->col_list.reserve(sizeof(int) * (size_t)(t->ncols + 4) + 16)) return rc;
-    unsigned long long *n_list = tm->col_list.as<unsigned long long>();
-    int *list = reinterpret_cast<int *>(n_list + 2);
-    cudaStream_t st = ctx().stream;
-    MPB_CUDA(cudaMemsetAsync(n_list, 0, 16, st));
-    LaunchCfg L = make_cfg(o, t->ncols);
-    unsigned long long *bits64 = reinterpret_cast<unsigned long long *>(d_bits32);
-#define CALLC(DW_, K_)                                                                                         \
-    do {                                                                                                       \
-        if (int rc = prep_kernel(classify_columns<DW_, K_>, L.smem)) return rc;                                \
-        classify_columns<DW_, K_><<<L.grid, kThreads, L.smem, st>>>(dV, t->colptr.as<int64_t>(), t->ncols, t->col0, \
-                                                                    t->r, S, L.table, L.words, L.M, L.use_smem, \
-                                                                    bits64, d_checks, list, n_list,            \
-                                                                    t->has_order ? t->col_order.as<int>() : nullptr); \
-    } while (0)
-    if (o->kind == 0) {
-        if (dw != 2) return fail(MPB200_EARG, "2-D obstacles need a 2-D workspace");
-        CALLC(2, 0);
-    } else {
-        switch (dw) {
-        case 1: CALLC(1, 1); break; case 2: CALLC(2, 1); break; case 3: CALLC(3, 1); break; case 4: CALLC(4, 1); break;
-        case 5: CALLC(5, 1); break; case 6: CALLC(6, 1); break; case 7: CALLC(7, 1); break; case 8: CALLC(8, 1); break;
-        case 9: CALLC(9, 1); break; case 10: CALLC(10, 1); break;
-        default: return edges_free_device_cols(dV, d, t, o, S, d_bits32, d_checks, nullptr, t->ncols);
-        }
-    }
-#undef CALLC
-    MPB_LAUNCHED();
-    return edges_free_device_cols(dV, d, t, o, S, d_bits32, d_checks, list, -1, n_list);
-}
-
-int edges_free_device_cols(const double *dV, int d, const mpb200_table *t, const mpb200_obstacles *o,
-                           const SpaceDev &S, uint32_t *d_bits32, unsigned long long *d_checks, const int *col_list,
-                           int64_t n_list, const unsigned long long *n_list_dev) {
-    const int dw = S.dw;
-    (void)d;
-    if (int rc = check_obstacles(o, dw)) return rc;
-    LaunchCfg L = make_cfg(o, (n_list_dev ? t->ncols : n_list) * 32);
-    cudaStream_t st = ctx().stream;
+    const double *dV = s->V.as<double>();
     const int64_t *colptr = t->colptr.as<int64_t>();
     const int64_t *rowval = t->rowval.as<int64_t>();
+    LaunchCfg L = make_cfg(o, t->ncols);
+    cudaStream_t st = ctx().stream;
+    static const bool no_classify = getenv("MPB200_NO_CLASSIFY") != nullptr;
+    const bool classify = t->euclid && S.s2w_kind == 0 && t->ncols > 0 && t->ncols < INT_MAX && !no_classify &&
+                          (o->kind == 0 ? dw == 2 : (dw >= 2 && dw <= 10));
+    if (classify) {  // one lane per column, then one warp per column of the list
+        if (int rc = t->col_list.reserve(sizeof(int) * (size_t)(t->ncols + 1))) return rc;
+        const CellOrder co = (t->has_order && t->grid_build == s->grid_build) ? cell_order(s) : CellOrder{nullptr, nullptr, nullptr};
+        const int *order = t->has_order ? t->col_order.as<int>() : nullptr;
+        int *list = t->col_list.as<int>();
+#define CALLC(DW_, K_)                                                                                         \
+        do {                                                                                                   \
+            if (int rc = prep_kernel(classify_columns<DW_, K_>, L.smem)) return rc;                            \
+            if (int rc = resident_grid(classify_columns<DW_, K_>, L.smem, t->ncols, &L.grid)) return rc;       \
+            classify_columns<DW_, K_><<<L.grid, kThreads, L.smem, st>>>(dV, colptr, t->ncols, t->col0, t->r, S, \
+                                                                        L.table, L.words, L.M, L.use_smem, order, \
+                                                                        co, d_bits32, d_counters, list);       \
+            MPB_LAUNCHED();                                                                                    \
+            if (int rc = prep_kernel(edges_free_kernel<DW_, DW_, K_>, L.smem)) return rc;                      \
+            if (int rc = resident_grid(edges_free_kernel<DW_, DW_, K_>, L.smem, t->ncols * 32, &L.grid)) return rc; \
+            edges_free_kernel<DW_, DW_, K_><<<L.grid, kThreads, L.smem, st>>>(dV, colptr, rowval, t->ncols, t->col0, \
+                                                                              S, L.table, L.words, L.M, L.use_smem, \
+                                                                              d_bits32, d_counters, list,      \
+                                                                              d_counters + 1);                 \
+        } while (0)
+        if (o->kind == 0) {
+            CALLC(2, 0);
+        } else {
+            switch (dw) {
+            case 2: CALLC(2, 1); break; case 3: CALLC(3, 1); break; case 4: CALLC(4, 1); break;
+            case 5: CALLC(5, 1); break; case 6: CALLC(6, 1); break; case 7: CALLC(7, 1); break;
+            case 8: CALLC(8, 1); break; case 9: CALLC(9, 1); break; default: CALLC(10, 1); break;
+            }
+        }
+#undef CALLC
+        MPB_LAUNCHED();
+        return 0;
+    }
+    // one warp per column
 #define CALL(N_, DW_, K_)                                                                                  \
     do {                                                                                                   \
         if (int rc = prep_kernel(edges_free_kernel<N_, DW_, K_>, L.smem)) return rc;                       \
-        edges_free_kernel<N_, DW_, K_><<<L.grid, kThreads, L.smem, st>>>(dV, colptr, rowval, t->ncols, t->col0, \
-                                                                         t->nnz, S, L.table, L.words, L.M, \
-                                                                         L.use_smem, d_bits32, d_checks, col_list, \
-                                                                         n_list, n_list_dev);              \
+        if (int rc = resident_grid(edges_free_kernel<N_, DW_, K_>, L.smem, t->ncols * 32, &L.grid)) return rc; \
+        edges_free_kernel<N_, DW_, K_><<<L.grid, kThreads, L.smem, st>>>(dV, colptr, rowval, t->ncols, t->col0, S, \
+                                                                         L.table, L.words, L.M, L.use_smem, \
+                                                                         d_bits32, d_counters, nullptr, nullptr); \
     } while (0)
     MPB_DISPATCH_DIMS(S.n, dw, o->kind, CALL);
 #undef CALL

@@ -110,9 +110,10 @@ struct mpb200_table {
     mpb::DevBuf masks;     // per-query hit lists (one byte per hit, 64 B/query; scratch between count and fill)
     mpb::DevBuf edge_bits; // uint64 ceil(nnz/64): last mpb200_edges_free result
     mpb::DevBuf scratch;   // big-column spill etc.
-    mpb::DevBuf col_list;  // int32 ncols + counter: columns that need per-edge checks
+    mpb::DevBuf col_list;  // int32 ncols: columns classify_columns leaves for the per-edge test (scratch)
     mpb::DevBuf col_order; // int32 ncols: the shard's columns in grid-cell order (spatially coherent warps)
     bool has_order = false;
+    uint64_t grid_build = 0;  // the samples' grid build that made col_order (its cell-ordered copy matches while equal)
     bool edge_bits_valid = false;  // edge_bits describes the CURRENT table contents (cleared by every build)
     int64_t edge_bits_nnz = 0;
     int64_t src_N = -1;            // the sample set the table was built from (rowval addresses its samples)
@@ -132,7 +133,8 @@ struct mpb200_samples {
     mpb::DevBuf sorted_idx;  // int32 N   original index of the k-th point in cell order
     mpb::DevBuf sorted_pos;  // f64 d x N positions in cell order (AoS)
     mpb::DevBuf pt_order;    // int32 (q1-q0): the shard's samples (relative to q0) in grid-cell order, from the last grid build
-    bool pt_order_valid = false;
+    bool pt_order_valid = false;  // sorted_pos, sorted_idx, q_order and pt_order still hold the last grid build
+    uint64_t grid_build = 0;      // serial of the last grid build
     bool sorted_x = false;   // samples are non-decreasing along the first coordinate (checked once at create)
     mpb::DevBuf minmax;      // f64 2*d bounding box
     double h_bbox[32] = {};  // host copy of the bounding box (mins then maxs), read once at create

@@ -747,6 +747,7 @@ static int build_table(mpb200_samples *s, double r, mpb200_table *t) {
     if (int rc = t->col_order.reserve(sizeof(int) * (size_t)(nq + 1))) return rc;
     if (int rc = s->pt_order.reserve(sizeof(int) * (size_t)(nq + 1))) return rc;
     s->pt_order_valid = false;
+    s->grid_build = next_serial();
     t->has_order = false;
     int *hist = s->cell_fill.as<int>();
     int *cell_start = s->cell_start.as<int>();
@@ -915,6 +916,7 @@ static int build_table(mpb200_samples *s, double r, mpb200_table *t) {
     t->r = r;
     t->euclid = true;
     t->has_order = nq > 0;
+    t->grid_build = s->grid_build;
     s->pt_order_valid = nq > 0;
     return 0;
 }
