@@ -76,6 +76,7 @@ int64_t mpb200_launch_count(void);
 #define MPB200_OP_EDGES 2  /* mpb200_edges_free / mpb200_lq_edges_free */
 #define MPB200_OP_OTHER 3  /* mpb200_mc_collision_probability */
 #define MPB200_OP_PLAN 4   /* mpb200_gmt_plan: phase 1 = the planning kernel */
+#define MPB200_OP_PATH 5   /* mpb200_shortcut_paths: phase 1 visibility, phase 2 minimum */
 double mpb200_last_ms(int phase);
 double mpb200_last_ms_of(int op, int phase);
 
@@ -460,6 +461,44 @@ int mpb200_gmt_plan_lazy(const mpb200_samples *s, const mpb200_gmt_desc *desc, c
 int mpb200_gmt_plan_batch(const mpb200_samples *s, const mpb200_gmt_desc *descs, int64_t nq,
                           const mpb200_gmt_edges *edges, mpb200_gmt_result *res, int64_t *segment_checks,
                           int64_t *paths, int64_t path_cap, int64_t *trees, double *costs);
+
+/* ---- shortcutting planned paths: the cheapest collision-free route through a path's subdivided waypoints ----------
+ * Not the reference's shortcut / adaptive_shortcut! (postprocessors.jl, not in the tree): specified here, restated in
+ * tests/oracle_shortcut.py.  npaths >= 1 paths, each handled on its own: path q is the states Y[0..L-1] (AoS, d doubles
+ * each) at rows offsets[q] .. offsets[q+1]-1 of states_aos (offsets[0] = 0, L = offsets[q+1] - offsets[q] >= 1).
+ *   1. Nodes: M = (L-1) k + 1 with k = subdivisions.  Node i k is Y[i] bit for bit; for m = 1..k-1 node i k + m is
+ *      Y[i]_c + t (Y[i+1]_c - Y[i]_c) with t = (double)m / (double)k, every operation rounded on its own (no FMA).
+ *   2. Visibility: for every pair a < b, free(a, b) = is_free_motion(node a, node b) with straight waypoints, the
+ *      predicate of mpb200_segments_free / mpb200_edges_free: node a is bounds-checked, node b is not.
+ *      segment_checks[q] = pairs whose segment test ran (node a in bounds; the CC.count increment);
+ *      pairs[q] = M (M-1) / 2.
+ *   3. Cost: cost(a, b) = sqrt(sum_c (node a_c - node b_c)^2), summed in index order, no FMA (the r-ball table's value).
+ *   4. Minimum: best[0] = +0.0; for b = 1..M-1, best[b] = min over free(a, b) of best[a] + cost(a, b) (one FP64 add),
+ *      pred[b] = the smallest a attaining it (the longest jump: collinear subdivision nodes drop out when costs tie);
+ *      +inf when no a gives a finite value.
+ *   5. Output: best[M-1] finite: the nodes of the pred chain 0 .. M-1, costs[q] = best[M-1].  Otherwise (the path was
+ *      not free): the input path unchanged, costs[q] = +inf.  L = 1: the input state, cost 0, 0 pairs.
+ * Guarantees:
+ *   - If every consecutive motion of the input is free -- true of every fmtstar / gmtstar / gmtstar_batch solution under
+ *     the same obstacles and space, whose planner tested exactly those endpoints in that direction -- the output cost
+ *     is <= the input's edge costs summed in path order, which is the planner's C[goal] bit for bit (the input edges
+ *     are edges of the minimum's DAG with the same cost formula, and FP64 addition is monotone).
+ *   - Every consecutive motion of the output is free: calling again on the output is valid and never raises the cost.
+ *   - The outputs of path q are byte-identical whatever else is in the call, in whatever order, on whatever grid
+ *     (MPB200_SHORTCUT_GRID=<blocks> forces the visibility pass's grid, clamped to the co-resident maximum).
+ * Outputs: out_len[q] and costs[q] always; row q of out_states (npaths x out_cap x d) only when out_len[q] <= out_cap;
+ * pairs and segment_checks may be NULL.  Waits for its results.
+ * Rejected with MPB200_EARG before any launch: npaths < 1; NULL states, offsets, out_len or costs; offsets not strictly
+ * increasing from 0 (a path with L = 0); subdivisions < 1; a path with M > MPB200_SHORTCUT_MAX_NODES; NULL out_states
+ * with out_cap > 0; out_cap < 0; a (d, workspace) / obstacle combination mpb200_segments_free rejects.  MPB200_ENOMEM,
+ * without a launch, when the scratch cannot be reserved (per path M ceil(M / 32) 4 bytes of visibility bits, about M^2 / 8, plus 16 d + 12 bytes per node).
+ * Three launches per call whatever npaths, timed under MPB200_OP_PATH (phase 1: nodes and visibility; phase 2: the
+ * minimum and the output rows). */
+#define MPB200_SHORTCUT_MAX_NODES 32768
+int mpb200_shortcut_paths(const double *states_aos, const int64_t *offsets, int64_t npaths, int d,
+                          const mpb200_obstacles *o, const mpb200_space_desc *ss, int32_t subdivisions,
+                          double *out_states, int64_t out_cap, int64_t *out_len, double *costs,
+                          int64_t *pairs, int64_t *segment_checks);
 
 #ifdef __cplusplus
 }

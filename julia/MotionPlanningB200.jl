@@ -442,4 +442,29 @@ function gmtstar_batch_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, inits:
     [(res[q], paths[1:res[q].path_len, q], trees[:, q], costs[:, q], segs[q]) for q in 1:nq]
 end
 
+# ---- shortcutting planned paths (mpb200_shortcut_paths; include/mpb200.h, DESIGN.md section 10c) -------------------
+"""shortcut_paths_b200(paths, CC, sd; subdivisions = 4): for each path (a d x L matrix of states, e.g. statevec2mat of
+a solution's states), the cheapest collision-free route through its subdivided waypoints under CC and the space of sd,
+all paths in one device call.  Not the reference's shortcut / adaptive_shortcut! (postprocessors.jl): the cost is never
+above the path's own, and a path that is not free comes back unchanged with cost Inf.  Returns, per path, (states as a
+d x L' matrix, cost, pairs, segment tests run); the segment tests are added to CC.count.  Written out in full but not
+run: Julia is not installed where this binding was written."""
+function shortcut_paths_b200(paths::Vector{Matrix{Float64}}, CC::B200Checker, sd::SpaceDesc; subdivisions = 4)
+    n = length(paths); d = size(paths[1], 1); k = Int32(subdivisions)
+    offsets = zeros(Int64, n + 1)
+    for q in 1:n
+        offsets[q + 1] = offsets[q] + size(paths[q], 2)
+    end
+    Y = hcat(paths...)                                       # d x sum(L): AoS, path q at columns offsets[q]+1 ..
+    cap = maximum((size(p, 2) - 1) * k + 1 for p in paths)
+    out = Array(Float64, d, cap, n)                          # row q of the C layout = out[:, :, q]
+    out_len = zeros(Int64, n); costs = zeros(Float64, n); pairs = zeros(Int64, n); segs = zeros(Int64, n)
+    check(ccall((:mpb200_shortcut_paths, LIB), Cint,
+                (Ptr{Float64}, Ptr{Int64}, Int64, Cint, Ptr{Void}, Ref{SpaceDescC}, Int32, Ptr{Float64}, Int64,
+                 Ptr{Int64}, Ptr{Float64}, Ptr{Int64}, Ptr{Int64}),
+                Y, offsets, n, d, CC.h, sd.c, k, out, cap, out_len, costs, pairs, segs))
+    CC.count += sum(segs)
+    [(out[:, 1:out_len[q], q], costs[q], pairs[q], segs[q]) for q in 1:n]
+end
+
 end # module

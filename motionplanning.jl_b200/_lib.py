@@ -66,7 +66,7 @@ GMT_EDGES_STRAIGHT, GMT_EDGES_LQ, GMT_EDGES_CAR = 0, 1, 2  # mpb200_gmt_edges.ki
 
 
 # every symbol include/mpb200.h declares: name -> (restype, argtypes)
-OP_TABLE, OP_POINTS, OP_EDGES, OP_OTHER, OP_PLAN = 0, 1, 2, 3, 4  # mpb200_last_ms_of operation kinds
+OP_TABLE, OP_POINTS, OP_EDGES, OP_OTHER, OP_PLAN, OP_PATH = 0, 1, 2, 3, 4, 5  # mpb200_last_ms_of operation kinds
 
 SIGNATURES = {
     "mpb200_init": (ctypes.c_int, [ctypes.c_int]),
@@ -129,6 +129,8 @@ SIGNATURES = {
                                             c_vp]),
     "mpb200_gmt_plan_batch": (ctypes.c_int, [c_vp, P(GmtDesc), c_i64, P(GmtEdges), P(GmtResult), c_vp, c_vp, c_i64,
                                              c_vp, c_vp]),
+    "mpb200_shortcut_paths": (ctypes.c_int, [c_vp, c_vp, c_i64, ctypes.c_int, c_vp, P(SpaceDesc), c_i32, c_vp, c_i64,
+                                             c_vp, c_vp, c_vp, c_vp]),
 }
 
 _lib = None

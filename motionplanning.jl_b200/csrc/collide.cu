@@ -15,6 +15,7 @@
 #include "philox.cuh"
 #include "scan.cuh"
 #include "gmt.cuh"
+#include "shortcut.cuh"
 #include <climits>
 #include <cstdlib>
 
@@ -445,12 +446,16 @@ static int prep_kernel(K kernel, size_t smem) {
 // there are fewer than that many CTAs' worth of items.  Call after prep_kernel (it sets the shared-memory limit).
 template <class K>
 static int resident_grid(K kernel, size_t smem, int64_t items, unsigned *grid) {
-    static size_t cached_smem = ~size_t(0);  // per kernel: the occupancy query is a host call per launch otherwise
+    // the last answer per kernel signature, keyed by the kernel itself too: the instantiations of a template share one
+    // signature (hence these statics) but not their register use; the occupancy query is a host call per launch otherwise
+    static const void *cached_kernel = nullptr;
+    static size_t cached_smem = ~size_t(0);
     static int per_sm = 0;
-    if (smem != cached_smem) {
+    if (smem != cached_smem || (const void *)kernel != cached_kernel) {
         MPB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, kThreads, smem));
         if (per_sm < 1) per_sm = 1;
         cached_smem = smem;
+        cached_kernel = (const void *)kernel;
     }
     const int64_t cap = (int64_t)per_sm * ctx().sm_count;
     const int64_t blocks = ceil_div(items > 0 ? items : 1, kThreads);
@@ -688,6 +693,111 @@ int sample_free_device(const mpb200_obstacles *o, const mpb200_space_desc *ss, i
             return fail(MPB200_EARG, "no free state among %lld candidates: the free space is empty", (long long)cands);
     }
     *h_used = c.h_scalar[13];
+    return 0;
+}
+
+// ---- shortcutting planned paths, phase 1 (mpb200_shortcut_paths; shortcut.cu runs the minimum) ----------------------
+// Row b of a path holds free(a, b) = motion_free(node a, node b) for every a < b.  One warp per row: node b's workspace
+// image stays in registers while the lanes take the nodes a < b 32 at a time (coalesced), with the warp-collective
+// segment test of column_edges; each ballot is one whole word of the row (a0 is a multiple of 32), so no atomics and no
+// memset.  The rows of every path form one flat list (global row = global node) dealt to the warps of a resident grid in
+// turn, so long and short paths share the warps.  Segment tests are summed per warp and flushed with one atomicAdd per
+// path the warp leaves.
+template <int N, int DW, int KIND>
+__global__ void __launch_bounds__(kThreads, (KIND == 0 || DW <= 4) ? 2 : 1)
+shortcut_visibility_kernel(const ShortcutPath *__restrict__ paths, int npaths, int64_t nrows,
+                           const double *__restrict__ nodes, SpaceDev S, const double *__restrict__ g_table,
+                           int table_words, int M, bool use_smem, uint32_t *__restrict__ bits,
+                           ShortcutResult *__restrict__ results) {
+    extern __shared__ double s_table[];
+    const double *T = stage_table(g_table, table_words, use_smem, s_table);
+    const int lane = threadIdx.x & 31;
+    const int64_t gwarp = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int64_t nwarps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+    Obs2 O(KIND == 0 ? T : nullptr, KIND == 0);
+    const LaneCull cl = lane_cull<KIND>(O);
+    int cur = -1;
+    unsigned long long my_checks = 0;  // lane 0: segment tests of path `cur` not yet added
+    for (int64_t g = gwarp; g < nrows; g += nwarps) {
+        const int q = shortcut_path_of(paths, npaths, g);
+        if (q != cur) {
+            if (lane == 0 && my_checks) atomicAdd(&results[cur].checks, my_checks);
+            my_checks = 0;
+            cur = q;
+        }
+        const int64_t node0 = paths[q].node0, bit0 = paths[q].bit0;
+        const int words = paths[q].words;
+        const int b = (int)(g - node0);
+        double w[N], qw[DW];
+#pragma unroll
+        for (int k = 0; k < N; ++k) w[k] = nodes[g * N + k];
+        state2workspace<N, DW>(S, w, qw);  // the last waypoint is never bounds-checked (Q4)
+        uint32_t *row = bits + bit0 + (int64_t)b * words;
+        const double *pv = nodes + node0 * N;
+        for (int a0 = 0; a0 < b; a0 += 32) {
+            const int a = a0 + lane;
+            bool run = false;
+            double v[N], p[DW];
+#pragma unroll
+            for (int k = 0; k < N; ++k) v[k] = 0.0;
+            if (a < b) {
+#pragma unroll
+                for (int k = 0; k < N; ++k) v[k] = pv[(int64_t)a * N + k];
+                run = in_state_space<N>(S, v);  // statespaces.jl:155: in_state_space(wps[1]) && segment test
+            }
+            state2workspace<N, DW>(S, v, p);
+            // warp-collective: every lane must make the call (no short-circuit on `run`)
+            bool seg_free;
+            if (KIND == 0)
+                seg_free = !warp_line_colliding_2d(O, cl.xl, cl.xh, cl.yl, cl.yh, p[0], p[DW > 1 ? 1 : 0], qw[0],
+                                                   qw[DW > 1 ? 1 : 0], run);
+            else
+                seg_free = warp_box_segment_free<DW>(T, M, p, qw, run);
+            const unsigned m = __ballot_sync(0xffffffffu, run && seg_free);
+            const unsigned ran = __ballot_sync(0xffffffffu, run);
+            if (lane == 0) {
+                row[a0 >> 5] = m;
+                my_checks += (unsigned long long)__popc(ran);
+            }
+        }
+    }
+    if (lane == 0 && my_checks) atomicAdd(&results[cur].checks, my_checks);
+}
+
+// The checks mpb200_segments_free makes of the space and obstacles, without a launch.
+int shortcut_check_space(const mpb200_obstacles *o, const mpb200_space_desc *ss, int d) {
+    SpaceDev S;
+    int dw = 0;
+    if (int rc = make_space(ss, d, &S, &dw)) return rc;
+    if (int rc = check_obstacles(o, dw)) return rc;
+#define CALL(N_, DW_, K_) do {} while (0)
+    MPB_DISPATCH_DIMS(S.n, dw, o->kind, CALL);
+#undef CALL
+    return 0;
+}
+
+int shortcut_visibility_device(const ShortcutPath *paths, int npaths, int64_t nodes_total, const double *nodes, int d,
+                               const mpb200_obstacles *o, const mpb200_space_desc *ss, uint32_t *bits,
+                               ShortcutResult *results) {
+    SpaceDev S;
+    int dw = 0;
+    if (int rc = make_space(ss, d, &S, &dw)) return rc;
+    if (int rc = check_obstacles(o, dw)) return rc;
+    LaunchCfg L = make_cfg(o, nodes_total);
+    cudaStream_t st = ctx().stream;
+    static const int env_grid = [] { const char *e = getenv("MPB200_SHORTCUT_GRID"); return e ? atoi(e) : 0; }();
+#define CALL(N_, DW_, K_)                                                                                        \
+    do {                                                                                                         \
+        if (int rc = prep_kernel(shortcut_visibility_kernel<N_, DW_, K_>, L.smem)) return rc;                    \
+        if (int rc = resident_grid(shortcut_visibility_kernel<N_, DW_, K_>, L.smem, nodes_total * 32, &L.grid))  \
+            return rc;                                                                                           \
+        if (env_grid > 0 && (unsigned)env_grid < L.grid) L.grid = (unsigned)env_grid;                            \
+        shortcut_visibility_kernel<N_, DW_, K_><<<L.grid, kThreads, L.smem, st>>>(                               \
+            paths, npaths, nodes_total, nodes, S, L.table, L.words, L.M, L.use_smem, bits, results);             \
+    } while (0)
+    MPB_DISPATCH_DIMS(S.n, dw, o->kind, CALL);
+#undef CALL
+    MPB_LAUNCHED();
     return 0;
 }
 

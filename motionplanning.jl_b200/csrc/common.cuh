@@ -13,7 +13,7 @@ namespace mpb {
 
 constexpr int kNumSMs = 148;  // B200: 2 dies x 74 SMs
 constexpr int kMaxPhases = 8;
-constexpr int kBanks = 5;  // separate phase-event banks: MPB200_OP_TABLE / _POINTS / _EDGES / _OTHER / _PLAN
+constexpr int kBanks = 6;  // separate phase-event banks: MPB200_OP_TABLE / _POINTS / _EDGES / _OTHER / _PLAN / _PATH
 
 struct Context {
     bool ready = false;

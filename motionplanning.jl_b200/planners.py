@@ -515,3 +515,66 @@ def gmtstar_batch(P, inits, goals, lam=1.0, N=None, rm=1.0, connections="R", r=0
         out[q] = MPSolution("solved" if rq.solved else "failed", float(rq.cost), elapsed, meta)
     CC.count = total_checks
     return out
+
+
+def shortcut_paths(P, paths=None, subdivisions=4):
+    """The cheapest collision-free route through each path's subdivided waypoints (mpb200_shortcut_paths) -> [dict]
+
+    paths: a list whose items are either a 1-D sequence of 1-based sample indices into P.V (the "path" of any solution,
+    including each gmtstar_batch result) or an (L, d) array of states; default [P.solution.metadata["path"]].  Each
+    edge is cut into `subdivisions` pieces; over the resulting waypoints, every pair a < b whose straight motion is free
+    under P.CC and P.SS is an edge of a DAG with the Euclidean cost, and the cheapest route from the first to the last
+    waypoint comes back (ties to the longest jump).  Not the reference's shortcut / adaptive_shortcut!: specified in
+    include/mpb200.h and DESIGN.md section 10c.  For a planner's solution under the same P.CC and P.SS the returned cost
+    is never above the planned one, and shortcutting a result again never raises its cost.  A path that is not free
+    comes back unchanged with cost inf.
+    Per path: {"states": (L', d) array, "cost": float, "pairs": waypoint pairs, "segment_checks": segment tests run};
+    the segment tests are added to P.CC.count, as segments_free does.  All paths go to the device in one call."""
+    from . import _lib
+    import ctypes
+
+    SS, CC = P.SS, P.CC
+    if not isinstance(SS.dist, Euclidean):
+        raise ValueError("shortcut_paths needs straight-line motions: Reeds-Shepp, Dubins and linear-quadratic spaces "
+                         "connect states by curves whose cost is defined only up to the steering radius")
+    if int(subdivisions) != subdivisions or subdivisions < 1:
+        raise ValueError("subdivisions must be an integer >= 1")
+    if paths is None:
+        sol = getattr(P, "solution", None)
+        if sol is None or sol.status != "solved":
+            raise ValueError("P has no solved path to shortcut")
+        paths = [sol.metadata["path"]]
+    d = SS.dim
+    V = P.V.V if hasattr(P.V, "V") else None
+    states = []
+    for p in paths:
+        a = np.asarray(p)
+        if a.ndim == 1 and a.size and np.issubdtype(a.dtype, np.integer):
+            if V is None or np.any(a < 1) or np.any(a > len(V)):
+                raise ValueError("path indices must be sample indices 1..N of P.V")
+            a = V[a - 1]
+        elif a.ndim == 2 and a.shape[0] >= 1 and a.shape[1] == d and np.issubdtype(a.dtype, np.number):
+            a = a.astype(np.float64)
+        else:
+            raise ValueError("each path must be non-empty: 1-based sample indices or an (L, %d) array of states" % d)
+        states.append(np.ascontiguousarray(a, dtype=np.float64))
+    n = len(states)
+    if n == 0:
+        raise ValueError("no paths given")
+    offsets = np.zeros(n + 1, dtype=np.int64)
+    offsets[1:] = np.cumsum([len(s) for s in states])
+    Y = np.ascontiguousarray(np.vstack(states))
+    k = int(subdivisions)
+    cap = max((len(s) - 1) * k + 1 for s in states)
+    out = np.empty((n, cap, d), dtype=np.float64)
+    out_len = np.empty(n, dtype=np.int64)
+    costs = np.empty(n, dtype=np.float64)
+    pairs = np.empty(n, dtype=np.int64)
+    segs = np.empty(n, dtype=np.int64)
+    space = SS.desc()
+    _lib.check(_lib.lib().mpb200_shortcut_paths(_lib.ptr(Y), _lib.ptr(offsets), n, d, CC.handle(), ctypes.byref(space),
+                                                k, _lib.ptr(out), cap, _lib.ptr(out_len), _lib.ptr(costs),
+                                                _lib.ptr(pairs), _lib.ptr(segs)))
+    CC.count += int(segs.sum())
+    return [{"states": out[q, :out_len[q]].copy(), "cost": float(costs[q]), "pairs": int(pairs[q]),
+             "segment_checks": int(segs[q])} for q in range(n)]
