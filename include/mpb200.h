@@ -462,6 +462,48 @@ int mpb200_gmt_plan_batch(const mpb200_samples *s, const mpb200_gmt_desc *descs,
                           const mpb200_gmt_edges *edges, mpb200_gmt_result *res, int64_t *segment_checks,
                           int64_t *paths, int64_t path_cap, int64_t *trees, double *costs);
 
+/* ---- roadmap-optimal plans: exact shortest paths over the resident roadmap (PRM*) -----------------------------
+ * The inputs of mpb200_gmt_plan in table mode (desc->width is ignored); specification restated in
+ * tests/oracle_sssp.py, DESIGN.md section 10d.
+ *   1. Graph: each stored entry e of column x of bwd, with row y, is an edge y -> x of cost nzval[e] when its edge bit
+ *      is set, y != x, and free(x) (the point bit of x when checkpts, else true): the connections GMT* step 4 could
+ *      commit.
+ *   2. Cost: d(init) = +0.0; d(x) = the minimum over all paths init -> x of the left fold ((0 + w1) + w2) + ..., each +
+ *      one FP64 add rounded to nearest; +inf when x is unreachable.  d is the unique fixed point of
+ *      d(x) = min_e d(y) + w_e, reached by any relaxation order.
+ *   3. d* = min of d over the goal vertices.  goal = init when init is a goal vertex, else the goal vertex with the
+ *      smallest (d, index); solved iff d* < +inf.  The outputs cover R = { x : d(x) <= d* } (failed: every reachable
+ *      vertex, so an empty goal mask gives the whole shortest-path tree); outside R, cost +inf and parent 0.
+ *   4. Tight edges T: graph edges y -> x with d(y) + nzval[e] == d(x) and x in R; h(x) = the BFS depth of x from init
+ *      in T (every x in R is reached).  tree[x] = the row of the first entry in storage order of column x of bwd that
+ *      is in T with h(y) = h(x) - 1.  The parent chain is acyclic and the fold of nzval along it equals d bit for bit.
+ *   5. Outputs: solved, goal (1-based, 0 when failed), cost = d(goal) (+inf when failed), path_len = h(goal) + 1
+ *      (0 when failed), reached = |R|, levels = BFS levels of T (1 + max h over R), rounds = relaxation rounds of the
+ *      search.  path (written when path_len <= path_cap), tree (N int64, 1-based, 0 = none) and costs (N f64) as
+ *      mpb200_gmt_plan.  Every output is a function of the sets above: byte-identical across runs and grid sizes.
+ * fwd must hold the transpose of bwd (every entry (y, x) of bwd has x in column y of fwd): true of every table pair
+ * the planners build (r-ball, LQ and car F/B, k-nearest knn / mutual knn).
+ * Rejected with MPB200_EARG as mpb200_gmt_plan in table mode rejects (tables from another sample set, sharded tables,
+ * missing or stale edge bits on bwd, checkpts without full-range point bits, init out of range), and for NULL s, desc,
+ * res or goal_bits or NULL path with path_cap > 0.  MPB200_ENOMEM, without a launch, when the scratch of
+ * MPB200_SSSP_BYTES(N, path_cap) bytes cannot be reserved.  One cooperative launch per call, timed under
+ * MPB200_OP_PLAN, grid as mpb200_gmt_plan (MPB200_GMT_GRID honoured).  Waits for its results. */
+typedef struct {
+    int32_t solved;
+    int32_t grid_blocks;        /* blocks of the cooperative launch */
+    int64_t goal;               /* 1-based goal vertex, 0 when failed */
+    double cost;                /* d(goal), +inf when failed */
+    int64_t path_len;           /* h(goal) + 1, 0 when failed */
+    int64_t rounds;             /* relaxation rounds of the cost phase */
+    int64_t levels;             /* BFS levels of the parent phase */
+    int64_t reached;            /* |R| */
+} mpb200_sssp_result;
+#define MPB200_SSSP_BYTES(N, path_cap) \
+    (44 * (int64_t)(N) + 8 * ((int64_t)(path_cap) < (int64_t)(N) ? (int64_t)(path_cap) : (int64_t)(N)) + \
+     8 * (((int64_t)(N) + 63) / 64) + 160)
+int mpb200_sssp_plan(const mpb200_samples *s, const mpb200_gmt_desc *desc, mpb200_sssp_result *res, int64_t *path,
+                     int64_t path_cap, int64_t *tree, double *costs);
+
 /* ---- shortcutting planned paths: the cheapest collision-free route through a path's subdivided waypoints ----------
  * Not the reference's shortcut / adaptive_shortcut! (postprocessors.jl, not in the tree): specified here, restated in
  * tests/oracle_shortcut.py.  npaths >= 1 paths, each handled on its own: path q is the states Y[0..L-1] (AoS, d doubles

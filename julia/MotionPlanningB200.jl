@@ -389,6 +389,35 @@ function gmtstar_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::BitVec
     r, path[1:r.path_len], tree, costs
 end
 
+# ---- PRM* on the device: mpb200_sssp_plan, the shortest path over the same tables and bits --------------------
+# C layout of mpb200_sssp_result (include/mpb200.h); the descriptor is GmtDescC, whose width is ignored.
+immutable SsspResultC
+    solved::Int32
+    grid_blocks::Int32
+    goal::Int64
+    cost::Float64
+    path_len::Int64
+    rounds::Int64
+    levels::Int64
+    reached::Int64
+end
+"""The roadmap-optimal plan (PRM*) over device tables, with the arguments of gmtstar_b200 but no width: the cheapest
+path from sample 1 to the goal over every edge of tB whose bit is set.  tree and costs cover the vertices no costlier
+than the goal (all reachable ones when the plan fails); the others have parent 0 and cost Inf.  Returns (result, path,
+tree, costs)."""
+function prmstar_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::BitVector, sd::SpaceDesc; checkpts = true)
+    N = length(goal)
+    path = Vector{Int64}(N); tree = Vector{Int64}(N); costs = Vector{Float64}(N)
+    res = Ref{SsspResultC}()
+    desc = Ref(GmtDescC(tF, tB, pointer(goal.chunks), 1, 0.0, Int32(checkpts),
+                        Base.unsafe_convert(Ptr{SpaceDescC}, sd.c)))        # goal and sd stay rooted by the arguments
+    check(ccall((:mpb200_sssp_plan, LIB), Cint,
+                (Ptr{Void}, Ref{GmtDescC}, Ref{SsspResultC}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}),
+                s.h, desc, res, path, N, tree, costs))
+    r = res[]
+    r, path[1:r.path_len], tree, costs
+end
+
 # C layout of mpb200_gmt_edges (include/mpb200.h): the motion check lazy GMT* runs on the one entry each candidate uses
 const GMT_EDGES_STRAIGHT = Int32(0)
 const GMT_EDGES_LQ = Int32(1)

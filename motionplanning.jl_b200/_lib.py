@@ -62,6 +62,11 @@ class GmtEdges(ctypes.Structure):
                 ("turning_radius", c_dbl), ("speed", c_dbl)]
 
 
+class SsspResult(ctypes.Structure):
+    _fields_ = [("solved", c_i32), ("grid_blocks", c_i32), ("goal", c_i64), ("cost", c_dbl), ("path_len", c_i64),
+                ("rounds", c_i64), ("levels", c_i64), ("reached", c_i64)]
+
+
 GMT_EDGES_STRAIGHT, GMT_EDGES_LQ, GMT_EDGES_CAR = 0, 1, 2  # mpb200_gmt_edges.kind
 
 
@@ -129,6 +134,7 @@ SIGNATURES = {
                                             c_vp]),
     "mpb200_gmt_plan_batch": (ctypes.c_int, [c_vp, P(GmtDesc), c_i64, P(GmtEdges), P(GmtResult), c_vp, c_vp, c_i64,
                                              c_vp, c_vp]),
+    "mpb200_sssp_plan": (ctypes.c_int, [c_vp, P(GmtDesc), P(SsspResult), c_vp, c_i64, c_vp, c_vp]),
     "mpb200_shortcut_paths": (ctypes.c_int, [c_vp, c_vp, c_i64, ctypes.c_int, c_vp, P(SpaceDesc), c_i32, c_vp, c_i64,
                                              c_vp, c_vp, c_vp, c_vp]),
 }

@@ -11,7 +11,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libmpb200.so")
-SOURCES = ["api.cu", "grid_rball.cu", "collide.cu", "lq.cu", "mc.cu", "brute_rball.cu", "tc_rball.cu", "order.cu", "xchg.cu", "peaks.cu", "lq_general.cu", "closest.cu", "knn.cu", "cars.cu", "gmt.cu", "gmt_lqg.cu", "shortcut.cu"]
+SOURCES = ["api.cu", "grid_rball.cu", "collide.cu", "lq.cu", "mc.cu", "brute_rball.cu", "tc_rball.cu", "order.cu", "xchg.cu", "peaks.cu", "lq_general.cu", "closest.cu", "knn.cu", "cars.cu", "gmt.cu", "gmt_lqg.cu", "shortcut.cu", "sssp.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -51,6 +51,24 @@ int gmt_launch_kernel(const void *kernel, void **args, int *blocks) {
     return 0;
 }
 
+int gmt_check_roadmap(const mpb200_samples *s, const mpb200_gmt_desc *desc, bool edge_bits) {
+    const int64_t N = s->N;
+    MPB_CHECK_ARG(s->d <= kMaxDim, "state dimension out of range");
+    for (const mpb200_table *t : {desc->fwd, desc->bwd}) {
+        MPB_CHECK_ARG(t->src_serial == s->serial && t->src_N == N && t->src_d == s->d,
+                      "a table was not built from this sample set");
+        MPB_CHECK_ARG(t->col0 == 0 && t->ncols == N, "a table covers a query range other than [0, N) (sharded tables are not supported)");
+    }
+    const mpb200_table *B = desc->bwd;
+    if (edge_bits)
+        MPB_CHECK_ARG(B->nnz == 0 || (B->edge_bits_valid && B->edge_bits_nnz == B->nnz),
+                      "the backward table has no edge bits for its current contents");
+    MPB_CHECK_ARG(!desc->checkpts || s->point_bits_valid, "checkpts needs the point bits of all N samples of this set");
+    const mpb200_space_desc *ss = desc->space;
+    MPB_CHECK_ARG(!ss || (ss->n == s->d && ss->lo && ss->hi), "space dimension does not match the samples");
+    return 0;
+}
+
 // edges == NULL: table mode.  A single plan is the batch of one query.
 static int gmt_plan(const mpb200_samples *s, const mpb200_gmt_desc *descs, int64_t nq, const mpb200_gmt_edges *edges,
                     mpb200_gmt_result *res, int64_t *segment_checks, int64_t *paths, int64_t path_cap, int64_t *trees,
@@ -74,19 +92,9 @@ static int gmt_plan(const mpb200_samples *s, const mpb200_gmt_desc *descs, int64
         MPB_CHECK_ARG(descs[q].init >= 1 && descs[q].init <= N, "init out of range (1..N)");
         MPB_CHECK_ARG(descs[q].width >= 0, "width must be a non-negative number");
     }
-    MPB_CHECK_ARG(s->d <= kMaxDim, "state dimension out of range");
-    for (const mpb200_table *t : {desc->fwd, desc->bwd}) {
-        MPB_CHECK_ARG(t->src_serial == s->serial && t->src_N == N && t->src_d == s->d,
-                      "a table was not built from this sample set");
-        MPB_CHECK_ARG(t->col0 == 0 && t->ncols == N, "a table covers a query range other than [0, N) (sharded tables are not supported)");
-    }
+    if (int rc = gmt_check_roadmap(s, desc, edges == nullptr)) return rc;
     const mpb200_table *B = desc->bwd;
-    if (!edges)
-        MPB_CHECK_ARG(B->nnz == 0 || (B->edge_bits_valid && B->edge_bits_nnz == B->nnz),
-                      "the backward table has no edge bits for its current contents");
-    MPB_CHECK_ARG(!desc->checkpts || s->point_bits_valid, "checkpts needs the point bits of all N samples of this set");
     const mpb200_space_desc *ss = desc->space;
-    MPB_CHECK_ARG(!ss || (ss->n == s->d && ss->lo && ss->hi), "space dimension does not match the samples");
     if (edges) {
         MPB_CHECK_ARG(ss != nullptr, "lazy edge tests need desc->space");
         MPB_CHECK_ARG(edges->obstacles != nullptr, "obstacle handle is NULL");

@@ -359,6 +359,11 @@ __global__ void __launch_bounds__(kGmtThreads) gmt_kernel(const GmtArgs a, const
 // MPB200_GMT_GRID=<blocks> overrides, clamped to the co-resident maximum), timed under MPB200_OP_PLAN.
 int gmt_launch_kernel(const void *kernel, void **args, int *blocks);
 
+// The argument checks every planner over the resident roadmap shares (gmt.cu): state dimension, fwd and bwd built
+// from s over [0, N), current edge bits on bwd when edge_bits, point bits of all N samples when desc->checkpts, and
+// the space's dimension.  0 or MPB200_EARG with the message set.  The callers check NULL pointers, N and init first.
+int gmt_check_roadmap(const mpb200_samples *s, const mpb200_gmt_desc *desc, bool edge_bits);
+
 template <class Edge>
 int gmt_launch(const GmtArgs &a, const Edge &edge, int *blocks) {
     void *args[] = {const_cast<GmtArgs *>(&a), const_cast<Edge *>(&edge)};

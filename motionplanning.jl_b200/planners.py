@@ -517,6 +517,59 @@ def gmtstar_batch(P, inits, goals, lam=1.0, N=None, rm=1.0, connections="R", r=0
     return out
 
 
+def prmstar(P, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, init_idx=1, checkpts=True, seed=0, k=None):
+    """PRM*: the shortest path over the roadmap, planned on the device -> (status, cost, elapsed)
+
+    Sets the problem and the roadmap up exactly as gmtstar(edge_checks="table") does (sample_free, radius, steering,
+    tables, edge bits, point bits), then finds, in one cooperative kernel (mpb200_sssp_plan), the cheapest path from
+    sample init_idx to the goal region over every collision-free edge of the backward table: a cost no FMT*-family
+    planner over the same roadmap can beat.  The tree and costs come back for every vertex no costlier than the goal
+    (every reachable vertex when the plan fails); the others have parent 0 and cost inf.  Specification:
+    include/mpb200.h, DESIGN.md section 10d.  Metadata: "planner" = "PRMstar", "path", "tree", "costs", "r", "k",
+    "rounds", "levels", "reached", "device_ms" and the roadmap keys gmtstar reports."""
+    from . import _lib
+    import ctypes
+
+    t_start = time.perf_counter()
+    N = len(P.V) if N is None else N
+    P.CC.count = 0
+    _gmt_check_args(connections, [0.0], "table")
+    SS, CC = P.SS, P.CC
+    if r > 0:
+        setup_steering(SS, r)
+    if not states_free(P.init, CC, SS)[0]:
+        P.status = "failed"
+        P.solution = MPSolution(P.status, math.inf, time.perf_counter() - t_start, {})
+        return math.inf
+    rmap = _gmt_roadmap(P, N, rm, connections, r, ensure_goal_ct, checkpts, seed, k, False)
+    NN, DF, DB = rmap["NN"], rmap["DF"], rmap["DB"]
+    V = NN.V
+    if not np.all(V[init_idx - 1] == P.init):
+        raise RuntimeError("P.V[init_idx] must be the init state (fmt.jl:48-66)")
+    goal_chunks = _goal_chunks(V, P.goal, SS)
+    space = SS.desc()
+    desc = _lib.GmtDesc(DF.h, DB.h, _lib.ptr(goal_chunks), init_idx, 0.0, int(bool(checkpts)), ctypes.pointer(space))
+    res = _lib.SsspResult()
+    tree = np.empty(N, dtype=np.int64)
+    C = np.empty(N, dtype=np.float64)
+    path = np.empty(N, dtype=np.int64)
+    lib = _lib.lib()
+    _lib.check(lib.mpb200_sssp_plan(NN.handle(), ctypes.byref(desc), ctypes.byref(res), _lib.ptr(path), N,
+                                    _lib.ptr(tree), _lib.ptr(C)))
+    device_ms = lib.mpb200_last_ms_of(_lib.OP_PLAN, 0)
+    sol = [int(v) for v in path[:res.path_len]]
+    P.status = "solved" if res.solved else "failed"
+    meta = {
+        "radius_multiplier": rm, "num_samples": N, "cost": float(res.cost), "cumcost": [float(C[v - 1]) for v in sol],
+        "planner": "PRMstar", "solved": bool(res.solved), "tree": tree, "path": sol, "costs": C, "r": rmap["r"],
+        "k": (rmap["k"] if rmap["knn_mode"] else None), "connections": connections,
+        "precomputed_edge_checks": int(rmap["lookups_before"]), "rounds": int(res.rounds), "levels": int(res.levels),
+        "reached": int(res.reached), "device_ms": device_ms, "grid_blocks": int(res.grid_blocks),
+    }
+    P.solution = MPSolution(P.status, float(res.cost), time.perf_counter() - t_start, meta)
+    return P.status, P.solution.cost, P.solution.elapsed
+
+
 def shortcut_paths(P, paths=None, subdivisions=4):
     """The cheapest collision-free route through each path's subdivided waypoints (mpb200_shortcut_paths) -> [dict]
 
