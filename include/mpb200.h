@@ -486,8 +486,9 @@ int mpb200_gmt_plan_batch(const mpb200_samples *s, const mpb200_gmt_desc *descs,
  * Rejected with MPB200_EARG as mpb200_gmt_plan in table mode rejects (tables from another sample set, sharded tables,
  * missing or stale edge bits on bwd, checkpts without full-range point bits, init out of range), and for NULL s, desc,
  * res or goal_bits or NULL path with path_cap > 0.  MPB200_ENOMEM, without a launch, when the scratch of
- * MPB200_SSSP_BYTES(N, path_cap) bytes cannot be reserved.  One cooperative launch per call, timed under
- * MPB200_OP_PLAN, grid as mpb200_gmt_plan (MPB200_GMT_GRID honoured).  Waits for its results. */
+ * MPB200_SSSP_BYTES(N, path_cap) bytes cannot be reserved (a plan is the batch of one query of
+ * mpb200_sssp_plan_batch).  One cooperative launch per call, timed under MPB200_OP_PLAN, grid as mpb200_gmt_plan
+ * (MPB200_GMT_GRID honoured).  Waits for its results. */
 typedef struct {
     int32_t solved;
     int32_t grid_blocks;        /* blocks of the cooperative launch */
@@ -498,11 +499,32 @@ typedef struct {
     int64_t levels;             /* BFS levels of the parent phase */
     int64_t reached;            /* |R| */
 } mpb200_sssp_result;
-#define MPB200_SSSP_BYTES(N, path_cap) \
-    (44 * (int64_t)(N) + 8 * ((int64_t)(path_cap) < (int64_t)(N) ? (int64_t)(path_cap) : (int64_t)(N)) + \
-     8 * (((int64_t)(N) + 63) / 64) + 160)
+#define MPB200_SSSP_BYTES(N, path_cap) (MPB200_SSSP_BATCH_BYTES_PER_QUERY(N, path_cap) + 96)
 int mpb200_sssp_plan(const mpb200_samples *s, const mpb200_gmt_desc *desc, mpb200_sssp_result *res, int64_t *path,
                      int64_t path_cap, int64_t *tree, double *costs);
+
+/* A batch of PRM* queries over one roadmap: nq independent plans over the same samples, the same fwd / bwd tables (and
+ * edge bits), point bits and checkpts setting.  Query q has its own init and goal mask from descs[q]; width and space
+ * are ignored, as in mpb200_sssp_plan.  Every output of query q (res[q] but grid_blocks -- rounds, levels and reached
+ * included --, row q of paths, trees and costs) is byte-identical to what mpb200_sssp_plan returns for descs[q] alone
+ * over the same tables, whatever the other queries of the batch, their order or the grid size.  grid_blocks is that of
+ * the one launch.  The queries march in lockstep through one cooperative launch and share its grid barriers: each
+ * step runs the threshold moves of the queries whose list is empty, then one relaxation round of every query still
+ * searching; then the BFS levels of all queries run together (DESIGN.md section 10d).
+ * paths: nq x path_cap, row q = the path of query q, written only when its path_len <= path_cap (paths may be NULL
+ * when path_cap == 0); trees (int64) and costs (f64): nq x N each, row q = query q, may be NULL.
+ * Rejected with MPB200_EARG before any launch: everything mpb200_sssp_plan rejects, for every query; nq < 1; NULL
+ * descs or res; descs whose fwd, bwd or checkpts differ from those of descs[0]; NULL paths with path_cap > 0.
+ * MPB200_ENOMEM, without a launch, when the scratch of the batch cannot be reserved: nq x
+ * MPB200_SSSP_BATCH_BYTES_PER_QUERY(N, path_cap) bytes of device memory (D, Dn, tree, two (query, vertex) lists: 8 N
+ * each; depth, stamp, pending flag: 4 N each; the path row, the goal mask, the 120-byte control block) plus 96 bytes
+ * for the whole batch.  One launch per call, timed under MPB200_OP_PLAN, grid as mpb200_gmt_plan (never sized from
+ * nq).  Waits for its results. */
+#define MPB200_SSSP_BATCH_BYTES_PER_QUERY(N, path_cap) \
+    (52 * (int64_t)(N) + 8 * ((int64_t)(path_cap) < (int64_t)(N) ? (int64_t)(path_cap) : (int64_t)(N)) + \
+     8 * (((int64_t)(N) + 63) / 64) + 120)
+int mpb200_sssp_plan_batch(const mpb200_samples *s, const mpb200_gmt_desc *descs, int64_t nq,
+                           mpb200_sssp_result *res, int64_t *paths, int64_t path_cap, int64_t *trees, double *costs);
 
 /* ---- shortcutting planned paths: the cheapest collision-free route through a path's subdivided waypoints ----------
  * Not the reference's shortcut / adaptive_shortcut! (postprocessors.jl, not in the tree): specified here, restated in

@@ -417,6 +417,22 @@ function prmstar_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, goal::BitVec
     r = res[]
     r, path[1:r.path_len], tree, costs
 end
+"""prmstar_b200 for a batch of queries over the same tables (mpb200_sssp_plan_batch): query q runs from sample
+inits[q] to the goal mask goals[q], all in one device launch.  Each query's outputs equal those of its own
+prmstar_b200 plan.  Returns, per query, (result, path, tree, costs).  Written out in full but not run: Julia is not
+installed where this binding was written."""
+function prmstar_batch_b200(s::B200Samples, tF::Ptr{Void}, tB::Ptr{Void}, inits::Vector{Int64},
+                            goals::Vector{BitVector}, sd::SpaceDesc; checkpts = true)
+    nq = length(inits); N = length(goals[1])
+    descs = [GmtDescC(tF, tB, pointer(goals[q].chunks), inits[q], 0.0, Int32(checkpts),
+                      Base.unsafe_convert(Ptr{SpaceDescC}, sd.c)) for q in 1:nq]   # goals and sd stay rooted
+    res = Vector{SsspResultC}(nq)
+    paths = Matrix{Int64}(N, nq); trees = Matrix{Int64}(N, nq); costs = Matrix{Float64}(N, nq)   # column q = query q
+    check(ccall((:mpb200_sssp_plan_batch, LIB), Cint,
+                (Ptr{Void}, Ptr{GmtDescC}, Int64, Ptr{SsspResultC}, Ptr{Int64}, Int64, Ptr{Int64}, Ptr{Float64}),
+                s.h, descs, nq, res, paths, N, trees, costs))
+    [(res[q], paths[1:res[q].path_len, q], trees[:, q], costs[:, q]) for q in 1:nq]
+end
 
 # C layout of mpb200_gmt_edges (include/mpb200.h): the motion check lazy GMT* runs on the one entry each candidate uses
 const GMT_EDGES_STRAIGHT = Int32(0)

@@ -22,7 +22,7 @@ from .simplecars import (ChoppedMetric, ChoppedQuasiMetric, DubinsExact, DubinsQ
                          ReedsSheppMetricSpace, car_motions_free, car_steer_batch, steering_control)
 from .problems import (BallGoal, MPProblem, MPSolution, PointGoal, RectangleGoal, StateGoal, is_goal_pt,  # noqa: F401
                        sample_free, sample_free_goal, sample_goal)
-from .planners import fmtstar, gmtstar, gmtstar_batch, prmstar, shortcut_paths  # noqa: F401
+from .planners import fmtstar, gmtstar, gmtstar_batch, prmstar, prmstar_batch, shortcut_paths  # noqa: F401
 from . import montecarlo  # noqa: F401
 from .montecarlo import MCProblem, collision_probability  # noqa: F401
 from . import obstaclesets  # noqa: F401

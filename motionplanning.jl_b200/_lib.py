@@ -135,6 +135,7 @@ SIGNATURES = {
     "mpb200_gmt_plan_batch": (ctypes.c_int, [c_vp, P(GmtDesc), c_i64, P(GmtEdges), P(GmtResult), c_vp, c_vp, c_i64,
                                              c_vp, c_vp]),
     "mpb200_sssp_plan": (ctypes.c_int, [c_vp, P(GmtDesc), P(SsspResult), c_vp, c_i64, c_vp, c_vp]),
+    "mpb200_sssp_plan_batch": (ctypes.c_int, [c_vp, P(GmtDesc), c_i64, P(SsspResult), c_vp, c_i64, c_vp, c_vp]),
     "mpb200_shortcut_paths": (ctypes.c_int, [c_vp, c_vp, c_i64, ctypes.c_int, c_vp, P(SpaceDesc), c_i32, c_vp, c_i64,
                                              c_vp, c_vp, c_vp, c_vp]),
 }

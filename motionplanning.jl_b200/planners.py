@@ -570,6 +570,74 @@ def prmstar(P, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, init_id
     return P.status, P.solution.cost, P.solution.elapsed
 
 
+def prmstar_batch(P, inits, goals, N=None, rm=1.0, connections="R", r=0.0, ensure_goal_ct=1, checkpts=True, seed=0,
+                  k=None, trees=True):
+    """A batch of PRM* queries over one roadmap -> [MPSolution], one per query
+
+    The roadmap is set up exactly as prmstar sets it up (sample 1 = P.init, P.goal's goal samples, radius, steering,
+    tables, edge bits, point bits); then every query q, from sample inits[q] (1-based) to goals[q] (a goal object: its
+    mask is goal_mask), is planned in one cooperative launch (mpb200_sssp_plan_batch).  Each query's solution equals
+    what prmstar would return for it over the same roadmap; a query whose init sample is not free is "failed" without a
+    plan.  Metadata: prmstar's keys plus "query" (its position in the batch) and "batch_size"; "device_ms" is the time
+    of the batch's kernel.  trees=False skips the nq x N tree and cost copies ("tree", "costs" and "cumcost" are
+    None)."""
+    from . import _lib
+    import ctypes
+
+    t_start = time.perf_counter()
+    inits = [int(i) for i in inits]
+    goals = list(goals)
+    nq = len(inits)
+    if nq == 0 or len(goals) != nq:
+        raise ValueError("inits and goals must be non-empty and of the same length")
+    N = len(P.V) if N is None else N
+    P.CC.count = 0
+    _gmt_check_args(connections, [0.0], "table")
+    if not all(1 <= i <= N for i in inits):
+        raise ValueError("inits must be sample indices 1..N")
+    SS, CC = P.SS, P.CC
+    if r > 0:
+        setup_steering(SS, r)
+    rmap = _gmt_roadmap(P, N, rm, connections, r, ensure_goal_ct, checkpts, seed, k, False)
+    NN, DF, DB = rmap["NN"], rmap["DF"], rmap["DB"]
+    V = NN.V
+    free = states_free(V[np.asarray(inits) - 1], CC, SS)      # fmt.jl:24-29, per query
+    planned = [q for q in range(nq) if free[q]]
+    n = len(planned)
+    space = SS.desc()
+    chunks = [_goal_chunks(V, goals[q], SS) for q in planned]
+    descs = (_lib.GmtDesc * max(n, 1))()
+    for j, q in enumerate(planned):
+        descs[j] = _lib.GmtDesc(DF.h, DB.h, _lib.ptr(chunks[j]), inits[q], 0.0, int(bool(checkpts)),
+                                ctypes.pointer(space))
+    res = (_lib.SsspResult * max(n, 1))()
+    paths = np.empty((n, N), dtype=np.int64)                  # rows as gmtstar_batch: only path_len entries are written
+    tree = np.empty((n, N), dtype=np.int64) if trees else None
+    C = np.empty((n, N), dtype=np.float64) if trees else None
+    lib = _lib.lib()
+    device_ms = 0.0
+    if n:
+        _lib.check(lib.mpb200_sssp_plan_batch(NN.handle(), descs, n, res, _lib.ptr(paths), N, _lib.ptr(tree),
+                                              _lib.ptr(C)))
+        device_ms = lib.mpb200_last_ms_of(_lib.OP_PLAN, 0)
+    elapsed = time.perf_counter() - t_start
+    out = [MPSolution("failed", math.inf, elapsed, {"query": q, "batch_size": nq}) for q in range(nq)]
+    for j, q in enumerate(planned):
+        rq = res[j]
+        sol = [int(v) for v in paths[j, :rq.path_len]]
+        meta = {
+            "radius_multiplier": rm, "num_samples": N, "cost": float(rq.cost),
+            "cumcost": None if C is None else [float(C[j, v - 1]) for v in sol], "planner": "PRMstar",
+            "solved": bool(rq.solved), "tree": None if tree is None else tree[j], "path": sol,
+            "costs": None if C is None else C[j], "r": rmap["r"], "k": (rmap["k"] if rmap["knn_mode"] else None),
+            "connections": connections, "precomputed_edge_checks": int(rmap["lookups_before"]),
+            "rounds": int(rq.rounds), "levels": int(rq.levels), "reached": int(rq.reached), "device_ms": device_ms,
+            "grid_blocks": int(rq.grid_blocks), "query": q, "batch_size": nq,
+        }
+        out[q] = MPSolution("solved" if rq.solved else "failed", float(rq.cost), elapsed, meta)
+    return out
+
+
 def shortcut_paths(P, paths=None, subdivisions=4):
     """The cheapest collision-free route through each path's subdivided waypoints (mpb200_shortcut_paths) -> [dict]
 
